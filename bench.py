@@ -44,6 +44,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from
 
 ALG_BYTES_PER_ROW = 644.0          # TIME 4 B + VOLT 320 B in, VOLT 320 B out (SURVEY.md 8d)
 DIODES = 32
@@ -73,7 +74,15 @@ def parse():
                          "measurement, never the headline (which is FP64)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="night only: after the timed steps, write what the last one returned (rank 0's "
+                         "tables) as .npy files in DIR, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "gppd" or args.config != "night"):
+        ap.error("--dump-outputs writes the outputs of the night (--impl gppd --config night)")
+    return args
 
 
 # --------------------------------------------------------------------------
@@ -202,7 +211,10 @@ def generate_night(torch, gp, dev, nfiles, nrows, rank, plan=None, faint_repeat=
             pscale = torch.where(st == 3, 3.0, torch.where(st == 1, 0.2, 1.0)).to(torch.float64)
         wt = 6.283185 * t
         for grp in range(8):
-            phi_fc = torch.cumsum(0.02 * torch.randn(nrows, generator=g, device=dev, dtype=torch.float64), 0)
+            # the random walk is summed on the host: a floating-point cumsum on the GPU is not
+            # bitwise reproducible, and every run must see the same night
+            walk = 0.02 * torch.randn(nrows, generator=g, device=dev, dtype=torch.float64)
+            phi_fc = torch.cumsum(walk.cpu(), 0).to(dev)
             phi_fc = phi_fc + float(torch.rand(1, generator=g, device=dev)) * 6.28 - 3.14
             efc = torch.polar(torch.ones_like(phi_fc), phi_fc)
             fcch = 32 + grp
@@ -242,6 +254,30 @@ def cpu_reference_files(oracle, files, cores):
         ofs = None if fs is None else oracle.FaintStates(fs.timer1, fs.timer2, 1.0, 2.0)
         oracle.processmetrology(tu, v, mjd, offsets=off, faintparam=ofs, nthreads=cores)
     return time.perf_counter() - t0
+
+
+DUMP_ROWS = 131_072     # demodulated VOLT rows kept by --dump-outputs (40 MB) ...
+DUMP_FITS = 262_144     # ... and fits (14 MB of params and chi2): less than 64 MB in all
+
+
+def dump_outputs(path, out, params, chi2):
+    """--dump-outputs: what the resident path returned, as .npy files in `path`:
+    volt_out [R, 80] float32 (demodulated VOLT rows in table, row order), params [M, 6] and
+    chi2 [M] float64 (fits in table, window, diode order).  Beyond DUMP_ROWS rows or
+    DUMP_FITS fits, a fixed, seeded sample of them is kept, in that order."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+
+    def keep(a, cap, seed):
+        a = a.reshape(a.shape[0] * a.shape[1], -1)
+        if a.shape[0] > cap:
+            pick = np.sort(np.random.default_rng(seed).choice(a.shape[0], cap, replace=False))
+            a = a[torch.from_numpy(pick).to(a.device)]
+        return a.cpu().numpy()
+
+    np.save(os.path.join(path, "volt_out.npy"), keep(out, DUMP_ROWS, 0))
+    np.save(os.path.join(path, "params.npy"), keep(params, DUMP_FITS, 1))
+    np.save(os.path.join(path, "chi2.npy"), keep(chi2, DUMP_FITS, 1)[:, 0])
 
 
 # --------------------------------------------------------------------------
@@ -374,6 +410,8 @@ def main():
     passes_overlapped = h.pass_times(reset=True)
     h.enable_timing(False)
     launches = h.launches - launches0
+    if args.dump_outputs and rank == 0:     # before the regions below overwrite the buffers
+        dump_outputs(args.dump_outputs, out, params, chi2)
     # ---- per-pass kernel times: a second region of the same K steps with ONE launch
     # sequence per batch.  In the throughput region above the FAINT and the bright tables
     # run as two concurrent chains (gppd_set_split_chains, default on), whose kernels

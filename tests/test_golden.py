@@ -1,7 +1,9 @@
 """Committed golden vectors (tests/golden/golden_small.npz, written by
 tests/golden/make_golden.py from the CPU oracle -- the reference itself cannot run
 here, see the script's header): the oracle must keep reproducing them bit for bit, and
-the CUDA path is compared with them without any oracle call at run time."""
+the CUDA path is compared with them without any oracle call at run time.  The input
+tables come from the seeded generator and are checked against the SHA-256 stored with
+the vectors."""
 import os
 import sys
 
@@ -12,6 +14,8 @@ import fitref
 from conftest import make_case
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import make_golden  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -20,10 +24,10 @@ def golden():
 
 
 def _inputs(gp, golden, name):
-    tab = {"time_us": golden[f"{name}_time_us"], "volt": golden[f"{name}_volt"],
-           "mjd": float(golden[f"{name}_mjd"])}
-    t, z = gp.synthetic.to_complex(tab, gp.synthetic.stefan_centres())
     st = golden["faint_state"] if name == "faint" else None
+    tab = make_golden.small_inputs(gp, name, st)
+    assert np.array_equal(make_golden.input_digest(tab), golden[f"{name}_sha256"]), "generator drifted"
+    t, z = gp.synthetic.to_complex(tab, gp.synthetic.stefan_centres())
     return tab, t, z, st
 
 
@@ -78,8 +82,6 @@ def golden_full():
 
 
 def _full_inputs(gp, ora, name):
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import make_golden
     return make_golden, make_golden.full_size_inputs(gp, ora, make_case, name)
 
 
