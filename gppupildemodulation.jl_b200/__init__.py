@@ -14,5 +14,5 @@ from ._lib import GppdError, Handle, build, default_handle  # noqa: F401
 from .api import (D1, D2, D3, D4, FC, FT, HIGH, LOW, M_2PI, NORMAL, OFF, SC,  # noqa: F401
                   TRANSIENT, Diode, FaintStates, MetState, ModulationNoOffsets,
                   ModulationWithOffsets, Side, buildfaintparameters, buildstates,
-                  demodulateall, idx, process_table, processmetrology, read_stefan_file,
+                  demodulateall, ellipse_keys, ellipses, idx, process_table, processmetrology, read_stefan_file,
                   table_windows)

@@ -13,6 +13,8 @@ CSRC = os.path.join(_HERE, "csrc")
 
 OK = 0
 ONLYHIGH, FITOFFSETS, NO_RECENTER, KEEPRAW, BIG_ENDIAN, CENTER_EMPIRICAL, FP32 = 1, 2, 4, 8, 16, 32, 64
+CENTER_ELLIPSE = 128
+ELLIPSE_STRIDE = 6
 METHOD_AUTO, METHOD_DIRECT, METHOD_HARMONIC = 0, 1, 2
 INFO_STRIDE = 4
 TRACE_MAX = 160
@@ -100,6 +102,7 @@ def lib():
     L.gppd_file_drain.argtypes = [H]
     L.gppd_wait.argtypes = [H, C.c_int]
     L.gppd_centres.argtypes = [H, C.c_int, C.c_int64, _dp]
+    L.gppd_ellipses.argtypes = [H, C.c_int, C.c_int64, _dp, _i32p]
     L.gppd_set_split_chains.argtypes = [H, C.c_int]
     L.gppd_debug_harmonics.argtypes = [H, C.c_int, _dp, C.c_int64]
     L.gppd_num_slots.argtypes = [H]
@@ -123,7 +126,7 @@ def lib():
                  "gppd_demodulate_f64_dev", "gppd_file_submit", "gppd_file_wait", "gppd_file_write",
                  "gppd_file_drain",
                  "gppd_table_windows", "gppd_process_table_f32", "gppd_submit_table_f32",
-                 "gppd_submit_fits_rows", "gppd_centres", "gppd_debug_harmonics", "gppd_set_split_chains",
+                 "gppd_submit_fits_rows", "gppd_centres", "gppd_ellipses", "gppd_debug_harmonics", "gppd_set_split_chains",
                  "gppd_wait", "gppd_num_slots", "gppd_process_table_f32_dev",
                  "gppd_process_tables_f32_dev", "gppd_enable_timing",
                  "gppd_pass_times", "gppd_measure_fp64_peak"):

@@ -133,12 +133,13 @@ def buildstates(faintstates: FaintStates, timestamp, lag: int = 0, preswitchdela
 
 
 def _options(onlyhigh=False, fitoffsets=False, recenter=True, keepraw=False, init="auto",
-             method="auto", maxfun=0, empirical=False, groups=0, fp32=False) -> Options:
+             method="auto", maxfun=0, empirical=False, groups=0, fp32=False, ellipse=False) -> Options:
     o = Options()
     o.group_mask = int(groups) & 0xff
     o.flags = ((_lib.ONLYHIGH if onlyhigh else 0) | (_lib.FITOFFSETS if fitoffsets else 0) |
                (0 if recenter else _lib.NO_RECENTER) | (_lib.KEEPRAW if keepraw else 0) |
-               (_lib.CENTER_EMPIRICAL if empirical else 0) | (_lib.FP32 if fp32 else 0))
+               (_lib.CENTER_EMPIRICAL if empirical else 0) | (_lib.FP32 if fp32 else 0) |
+               (_lib.CENTER_ELLIPSE if ellipse else 0))
     o.method = {"auto": _lib.METHOD_AUTO, "direct": _lib.METHOD_DIRECT,
                 "harmonic": _lib.METHOD_HARMONIC}[method]
     o.maxfun = int(maxfun)
@@ -229,13 +230,19 @@ def table_windows(time_us, mjd, window):
 
 def process_table(time_us, volt, mjd, offsets=None, faintparam: FaintStates | None = None,
                   window=None, keepraw=False, onlyhigh=False, method="auto", maxfun=0,
-                  handle=None, centres_out=None, fp32=False):
+                  handle=None, centres_out=None, fp32=False, ellipses_out=None,
+                  ellipse_status_out=None):
     """Array-level fast path (C ABI ``gppd_process_table_f32``): returns
     (volt_out float32 (N, 80|144), params (nwin*32, 6), chi2, info, state|None).
     ``offsets``: (40,) complex128 centres, ``None`` (fit the centres) or ``True``
     (empirical circle centres, fitted on the device; ``centres_out``, a (40,)
     complex128 array, then receives them).  ``fp32=True`` (GPPD_FP32): the optional
-    reduced-precision harmonic sums; parameters within 1e-5 of the FP64 path."""
+    reduced-precision harmonic sums; parameters within 1e-5 of the FP64 path.
+    ``offsets="ellipse"`` (GPPD_CENTER_ELLIPSE): one least-squares ellipse per channel,
+    fitted on the device, maps every channel onto a circle before the fit (include/gppd.h);
+    ``ellipses_out`` ((40, 6) float64: x0, y0, r, alpha, m21, m22) and
+    ``ellipse_status_out`` ((40,) int32: 2 ellipse, 1 circle only, 0 neither) then receive
+    the maps."""
     h = handle or _lib.default_handle()
     tu = np.ascontiguousarray(time_us, dtype=np.int32)
     v = np.ascontiguousarray(volt, dtype=np.float32)
@@ -243,10 +250,14 @@ def process_table(time_us, volt, mjd, offsets=None, faintparam: FaintStates | No
     if v.shape != (n, 80):
         raise ValueError("VOLT must be (N, 80) float32")
     empirical = offsets is True
-    off = None if (offsets is None or empirical) else np.ascontiguousarray(offsets, dtype=np.complex128)
+    ellipse = isinstance(offsets, str) and offsets == "ellipse"
+    if isinstance(offsets, str) and not ellipse:
+        raise ValueError("offsets: (40,) centres, None, True or 'ellipse'")
+    off = (None if (offsets is None or empirical or ellipse)
+           else np.ascontiguousarray(offsets, dtype=np.complex128))
     _, nwin = table_windows(tu, mjd, window)
     o = _options(onlyhigh=onlyhigh, keepraw=keepraw, method=method, maxfun=maxfun,
-                 empirical=empirical, fp32=fp32)
+                 empirical=empirical, fp32=fp32, ellipse=ellipse)
     vout = np.empty((n, 144 if keepraw else 80), dtype=np.float32)
     params = np.empty((nwin * 32, 6))
     chi2 = np.empty(nwin * 32)
@@ -264,7 +275,40 @@ def process_table(time_us, volt, mjd, offsets=None, faintparam: FaintStates | No
         c = np.empty(40, dtype=np.complex128)
         check(lib().gppd_centres(h.raw, 0, 1, ptr(c.view(np.float64))))
         centres_out[:] = c
+    if ellipse and (ellipses_out is not None or ellipse_status_out is not None):
+        e, st = ellipses(h, 0, 1)
+        if ellipses_out is not None:
+            ellipses_out[:] = e[0]
+        if ellipse_status_out is not None:
+            ellipse_status_out[:] = st[0]
     return vout, params, chi2, info, state
+
+
+def ellipses(handle=None, slot=0, ntables=1):
+    """The maps of the last ``offsets="ellipse"`` call on pipeline slot ``slot``
+    (``gppd_ellipses``): (ell (ntables, 40, 6) = x0, y0, r, alpha, m21, m22,
+    status (ntables, 40) int32)."""
+    h = handle or _lib.default_handle()
+    e = np.empty((ntables, 40, _lib.ELLIPSE_STRIDE))
+    st = np.empty((ntables, 40), dtype=np.int32)
+    check(lib().gppd_ellipses(h.raw, int(slot), int(ntables), ptr(e), ptr(st, _lib._i32p)))
+    return e, st
+
+
+def ellipse_keys(ell) -> dict:
+    """Header keywords of ``--center ellipse``, the transform applied to VOLT:
+    DEMODULATION ELLIPSE {X0|Y0|RATIO|ANGLE} {FT|SC} T{1-4} {D1-D4|FC} (160 values) from
+    the (40, 6) maps of ``ellipses``."""
+    ell = np.asarray(ell, dtype=np.float64).reshape(40, 6)
+    hdr = {}
+    for s in (Side.FT, Side.SC):
+        for j in range(1, 5):
+            for d in (Diode.D1, Diode.D2, Diode.D3, Diode.D4, Diode.FC):
+                # idx() of src/Modulation.jl:17-22, 0-based (no library call: a header helper)
+                ch = 32 + s // 4 + (j - 1) if d == Diode.FC else s + (d - 1) + (j - 1) * 4
+                for q, k in (("X0", 0), ("Y0", 1), ("RATIO", 2), ("ANGLE", 3)):
+                    hdr[f"DEMODULATION ELLIPSE {q} {s.name} T{j} {d.name}"] = float(ell[ch, k])
+    return hdr
 
 
 def _rem2pi_nearest(x):
@@ -328,17 +372,21 @@ def processmetrology(table, mjd, window=None, faintparam: FaintStates | None = N
     empirical centres, ``compute_offsets`` :105-125 -- one least-squares circle per
     channel over the HIGH samples of a FAINT table, all samples otherwise.  The
     reference throws here because its ``Circle`` is undefined; this is the algebraic
-    circle fit that call stands for)."""
+    circle fit that call stands for) or ``"ellipse"`` (one ellipse per channel, see
+    ``process_table``; the header then records the maps, ``ellipse_keys``)."""
     out = dict(table)
     hdr = {}
-    if offsets is True:
+    ell = np.empty((40, 6)) if isinstance(offsets, str) and offsets == "ellipse" else None
+    if ell is not None:
+        off = "ellipse"
+    elif offsets is True:
         off = True
     else:
         off = None if offsets is False else np.asarray(offsets, dtype=np.complex128)
     fitoffsets = off is None
     vout, params, chi2, info, state = process_table(
         table["TIME"], table["VOLT"], mjd, offsets=off, faintparam=faintparam, window=window,
-        keepraw=keepraw, onlyhigh=onlyhigh, handle=handle, method=method)
+        keepraw=keepraw, onlyhigh=onlyhigh, handle=handle, method=method, ellipses_out=ell)
     n = vout.shape[0]
     if window is None:
         hdr.update(demodulation_keys(params, fitoffsets))
@@ -347,6 +395,8 @@ def processmetrology(table, mjd, window=None, faintparam: FaintStates | None = N
         out.update(window_columns(params, n, wrows, nwin, fitoffsets))
         if state is not None:
             out["STATE"] = state.astype(np.int8)   # :248
+    if ell is not None:
+        hdr.update(ellipse_keys(ell))
     hdr["PROCSOFT"] = "GPPupilDemodulation.jl"     # :252
     out["VOLT"] = vout                             # :253
     return out, hdr

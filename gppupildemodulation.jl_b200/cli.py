@@ -36,8 +36,8 @@ import numpy as np
 
 from . import _lib, fits
 from .sharding import partition_files
-from .api import (_options, buildfaintparameters, demodulation_keys, read_stefan_file,
-                  window_columns)
+from .api import (_options, buildfaintparameters, demodulation_keys, ellipse_keys, ellipses,
+                  read_stefan_file, window_columns)
 
 SUFFIXES = (".fits", ".fits.gz", "fits.Z")      # src/GPPupilDemodulation.jl:14
 log = logging.getLogger("GPPupilDemodulation")
@@ -57,7 +57,8 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--verbose", "-v", action="store_true", help="Verbose mode")
     p.add_argument("--keepraw", "-k", action="store_true", help="keep raw")
     p.add_argument("--center", "-c", default="stefan",
-                   help="center voltages: stefan (default) | empirical | uncentered | fit")
+                   help="center voltages: stefan (default) | empirical | uncentered | fit | ellipse "
+                        "(offset and ellipse correction of each channel, fitted per file)")
     p.add_argument("--window", "-w", type=float, default=0.0,
                    help="Compute demodulation on non overlapping window of WINDOW second")
     p.add_argument("--dir", "-d", default=os.getcwd(), help="output folder")
@@ -126,7 +127,9 @@ class NightScheduler:
     def __init__(self, handle, offsets, onlyhigh, method="auto"):
         self.h, self.L = handle, _lib.lib()
         self.empirical = offsets is True       # --center empirical: centres fitted on the device
-        self.offsets = (None if (offsets is None or self.empirical)
+        # --center ellipse: one ellipse per channel fitted and applied on the device
+        self.ellipse = isinstance(offsets, str) and offsets == "ellipse"
+        self.offsets = (None if (offsets is None or self.empirical or self.ellipse)
                         else np.ascontiguousarray(offsets, dtype=np.complex128))
         self.onlyhigh, self.method = onlyhigh, method
         self.nslots = handle.num_slots
@@ -172,7 +175,7 @@ class NightScheduler:
             wrows = w.value
             nwin = (n + wrows - 1) // wrows
         o = _options(onlyhigh=self.onlyhigh, keepraw=job.keepraw, method=self.method,
-                     empirical=self.empirical)
+                     empirical=self.empirical, ellipse=self.ellipse)
         fp = job.faintparam
         t1 = fp.timer1 if fp is not None else None
         t2 = fp.timer2 if fp is not None else None
@@ -213,16 +216,23 @@ class NightScheduler:
         if job.native:
             return self._finish_native(slot, job, b)
         _lib.check(self.L.gppd_wait(self.h.raw, slot))
+        b["ell"] = self._ellipses(slot)
         # the slot's staging buffers are reused by the next file: take the results out
         b = dict(b, rows_out=b["rows_out"].copy(), params=b["params"].copy(), chi2=b["chi2"].copy(),
                  state=None if b["state"] is None else b["state"].copy())
         return self.writers.submit(self._write, job, b)
 
+    def _ellipses(self, slot):
+        """The (40, 6) maps of the slot's last file (--center ellipse), else None."""
+        return ellipses(self.h, slot, 1)[0][0] if self.ellipse else None
+
     def _table_edits(self, job, b, n):
         """(header keys, new columns, extra per-row bytes or None) of the output table
         (reference :174-189 whole-file keys, :209-249 window-mode columns)."""
-        fitoffsets = self.offsets is None and not self.empirical
+        fitoffsets = self.offsets is None and not self.empirical and not self.ellipse
         keys, newcols, extra = [], [], None
+        if self.ellipse:                    # the transform applied to VOLT, both modes
+            keys += list(ellipse_keys(b["ell"]).items())
         if job.window is None:
             keys += list(demodulation_keys(b["params"], fitoffsets).items())
         else:
@@ -248,6 +258,7 @@ class NightScheduler:
         b["state"] = np.empty(n, dtype=np.int8) if job.faintparam is not None else None
         _lib.check(self.L.gppd_file_wait(self.h.raw, slot, _lib.ptr(b["params"]), _lib.ptr(b["chi2"]), None,
                                          _lib.ptr(b["state"], _lib._i8p)))
+        b["ell"] = self._ellipses(slot)
         keys, newcols, extra = self._table_edits(job, b, n)
         met = job.hdus[job.imet]
         rb_new = b["rb_out"] + (0 if extra is None else extra.shape[1])
@@ -350,6 +361,8 @@ def main(argv=None) -> int:
         offsets = True
     elif args.center == "fit":
         offsets = None
+    elif args.center == "ellipse":       # offset + ellipse (Heydemann) correction per channel
+        offsets = "ellipse"
     else:
         raise SystemExit(f"unknown --center {args.center}")
     mine = partition_files(files, args.rank, args.world)   # no communication between ranks

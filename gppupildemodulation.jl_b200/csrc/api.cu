@@ -155,6 +155,11 @@ struct Slot {
     long long htab_vals = 0;        // values in htab after the last batch (test hook)
     DevBuf centres, cpart;          // --center empirical: [T][40] complex128 + partial sums
     int ncentres = 0;               // tables whose centres the last batch of this slot fitted
+    // --center ellipse: descriptors, [T][40][6] maps + [T][40] statuses, partial sums, and the
+    // complex128 arrays between the correction and the repack (t, corrected data, demodulated
+    // out, FAINT states when the caller keeps none)
+    DevBuf etabs, ell, estatus, epart, et, edata, eout, estate;
+    int nellipses = 0;              // tables whose ellipses the last batch of this slot fitted
     DevBuf params, chi2, info, trace, state_out;
     // batch scratch
     DevBuf state, basis, z, y, thkeys, nvalid, jobs, results;
@@ -480,6 +485,7 @@ int run_batch(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs
     }
 
     s.ncentres = 0;
+    if (!segment_only) s.nellipses = 0;
     if (empirical) {
         // offsets === true: every table gets its own 40 centres, fitted on the device
         if ((rc = s.centres.ensure(sizeof(double2) * NCHAN * (size_t)T))) return rc;
@@ -630,8 +636,11 @@ int check_handle(gppd_handle h) {
 }
 
 // offsets of processmetrology (src/GPPupilDemodulation.jl:150-157): a vector => subtract it;
-// true (GPPD_CENTER_EMPIRICAL) => circle centres fitted here; false (NULL) => fitoffsets
+// true (GPPD_CENTER_EMPIRICAL) => circle centres fitted here; false (NULL) => fitoffsets.
+// GPPD_CENTER_ELLIPSE ignores the vector and keeps the caller's flags (run_batch_ellipse
+// refuses GPPD_FITOFFSETS and GPPD_CENTER_EMPIRICAL with it).
 void centre_mode(gppd_options &o, bool have_offsets) {
+    if (o.flags & GPPD_CENTER_ELLIPSE) return;
     if (o.flags & GPPD_CENTER_EMPIRICAL) o.flags &= ~GPPD_FITOFFSETS;
     else if (!have_offsets) o.flags |= GPPD_FITOFFSETS;
     else o.flags &= ~GPPD_FITOFFSETS;
@@ -655,6 +664,133 @@ void table_views(int64_t n, double mjd, const int32_t *d_time, const float *d_vo
     a.ov.keepraw = (flags & GPPD_KEEPRAW) ? 1 : 0;
     a.ov.volt = d_volt_out;
     a.ov.volt_stride = a.ov.keepraw ? 576 : 320;
+}
+
+// `--center ellipse` on a batch of kind-0 tables: a composition of existing passes around the
+// ellipse kernels (centre_kernels.cu), all on `stream`:
+//   1. FAINT segmentation of the tables that have timers (run_batch, segment_only)
+//   2. moments + conic solve per channel -> s.ell / s.estatus      (GPPD_PASS_BASIS)
+//   3. the correction: TIME + VOLT rows -> t, data[40][n] complex128 (GPPD_PASS_BASIS)
+//   4. the array path of gppd_demodulate_f64_dev on (t, data, states) -> out[40][n]
+//   5. the repack of out into the caller's VOLT rows               (GPPD_PASS_DEMOD)
+int run_batch_ellipse(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs> &tabs,
+                      const gppd_options &o) {
+    if (o.flags & (GPPD_CENTER_EMPIRICAL | GPPD_FITOFFSETS)) {
+        g_last_error = "GPPD_CENTER_ELLIPSE excludes GPPD_CENTER_EMPIRICAL and GPPD_FITOFFSETS";
+        return GPPD_ERR_ARG;
+    }
+    if ((o.group_mask & 0xffu) != 0 && (o.group_mask & 0xffu) != 0xffu) {
+        g_last_error = "gppd_options.group_mask: a partial mask applies to the demodulate_f64 entry points only";
+        return GPPD_ERR_UNSUPPORTED;
+    }
+    const int T = (int)tabs.size();
+    if (T <= 0) return GPPD_OK;
+    long long R = 0, max_rows = 0, R_state = 0;
+    for (const TableArgs &a : tabs) {
+        if (a.tv.kind != 0 || a.tv.n < 2) {
+            g_last_error = "GPPD_CENTER_ELLIPSE: need METROLOGY tables of at least 2 rows";
+            return GPPD_ERR_ARG;
+        }
+        R += a.tv.n;
+        if (a.tv.n > max_rows) max_rows = a.tv.n;
+        if (a.n1 > 0 && a.n2 > 0 && !a.d_state_out) R_state += a.tv.n;
+    }
+    const int P = circle_max_segments(max_rows);
+    int rc;
+    if ((rc = s.etabs.ensure(sizeof(TableDesc) * (size_t)T))) return rc;
+    if ((rc = s.ell.ensure(sizeof(double) * ELL_STRIDE * NCHAN * (size_t)T))) return rc;
+    if ((rc = s.estatus.ensure(sizeof(int) * NCHAN * (size_t)T))) return rc;
+    if ((rc = s.epart.ensure(sizeof(double) * ELL_VALS * NCHAN * (size_t)T * (size_t)P))) return rc;
+    if ((rc = s.et.ensure(sizeof(double) * (size_t)R))) return rc;
+    if ((rc = s.edata.ensure(sizeof(double2) * NCHAN * (size_t)R))) return rc;
+    if ((rc = s.eout.ensure(sizeof(double2) * NCHAN * (size_t)R))) return rc;
+    if (R_state)
+        if ((rc = s.estate.ensure((size_t)R_state))) return rc;
+
+    // 1. states of the FAINT tables (into the caller's buffer when there is one)
+    std::vector<TableArgs> seg;
+    std::vector<int8_t *> states((size_t)T, nullptr);
+    {
+        size_t st_off = 0;
+        for (int t = 0; t < T; ++t) {
+            TableArgs &a = tabs[t];
+            if (!(a.n1 > 0 && a.n2 > 0)) continue;
+            if (!a.d_state_out) {
+                a.d_state_out = s.estate.as<int8_t>() + st_off;
+                st_off += (size_t)a.tv.n;
+            }
+            states[t] = a.d_state_out;
+            seg.push_back(a);
+        }
+    }
+    if (!seg.empty())
+        if ((rc = run_batch(h, s, stream, seg, nullptr, nullptr, true))) return rc;
+
+    // 2. + 3. the ellipses and the corrected arrays
+    std::vector<TableDesc> td((size_t)T);
+    std::vector<TableArgs> arr((size_t)T);
+    {
+        size_t row_off = 0;
+        for (int t = 0; t < T; ++t) {
+            const TableArgs &a = tabs[t];
+            TableDesc &d = td[t];
+            memset(&d, 0, sizeof d);
+            d.tv = a.tv;
+            d.ov = a.ov;
+            d.tv.offsets = reinterpret_cast<const double2 *>(s.ell.as<double>() + (size_t)t * NCHAN * ELL_STRIDE);
+            d.tv.t = s.et.as<double>() + row_off;
+            d.tv.data = s.edata.as<double2>() + NCHAN * row_off;
+            d.ov.out = s.eout.as<double2>() + NCHAN * row_off;
+            d.state = states[t];
+            TableArgs &b = arr[t];
+            memset(&b.tv, 0, sizeof b.tv);
+            memset(&b.ov, 0, sizeof b.ov);
+            b.tv.kind = 1;
+            b.tv.n = a.tv.n;
+            b.tv.t = d.tv.t;
+            b.tv.data = d.tv.data;
+            b.ov.kind = 1;
+            b.ov.out = d.ov.out;
+            b.wrows = a.wrows;
+            b.d_state_in = states[t];
+            b.d_params = a.d_params;
+            b.d_chi2 = a.d_chi2;
+            b.d_info = a.d_info;
+            row_off += (size_t)a.tv.n;
+        }
+    }
+    // (small pageable copy: staged by the runtime before cudaMemcpyAsync returns)
+    CK(cudaMemcpyAsync(s.etabs.p, td.data(), sizeof(TableDesc) * (size_t)T, cudaMemcpyHostToDevice, stream));
+    const TableDesc *d_tabs = s.etabs.as<TableDesc>();
+    Launcher L{stream, &h->launches};
+    {
+        PassScope ps(h, s, stream, GPPD_PASS_BASIS);
+        launch_ellipse_fit(L, d_tabs, T, max_rows, s.epart.as<double>(), s.ell.as<double>(), s.estatus.as<int>());
+        launch_ellipse_apply(L, d_tabs, T, max_rows, s.ell.as<double>());
+    }
+    DBG(stream, "ellipse");
+
+    // 4. the ordinary array path, NoOffsets model (GPPD_FP32 has no array form: no effect here)
+    gppd_options o4 = o;
+    o4.flags &= ~(GPPD_CENTER_ELLIPSE | GPPD_KEEPRAW | GPPD_BIG_ENDIAN | GPPD_FP32);
+    if ((rc = run_batch(h, s, stream, arr, &o4, nullptr, false))) return rc;
+
+    // 5. back to VOLT rows
+    {
+        PassScope ps(h, s, stream, GPPD_PASS_DEMOD);
+        launch_repack_arrays(L, d_tabs, T, max_rows, (o.flags & GPPD_KEEPRAW) != 0);
+    }
+    DBG(stream, "repack");
+    CK(cudaGetLastError());
+    s.nellipses = T;
+    return GPPD_OK;
+}
+
+// the batch of a table entry point: the ellipse composition or the ordinary launch sequence
+int run_tables(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs> &tabs,
+               const gppd_options &o) {
+    if (o.flags & GPPD_CENTER_ELLIPSE) return run_batch_ellipse(h, s, stream, tabs, o);
+    return run_batch(h, s, stream, tabs, &o, nullptr, false);
 }
 
 }  // namespace
@@ -758,6 +894,8 @@ int gppd_destroy(gppd_handle h) {
                           &s.timers, &s.lb, &s.events, &s.flags, &s.tabs, &s.exps, &s.faintjobs, &s.fbq,
                           &s.centres, &s.cpart};
         for (DevBuf *b : bufs) b->release();
+        DevBuf *ebufs[] = {&s.etabs, &s.ell, &s.estatus, &s.epart, &s.et, &s.edata, &s.eout, &s.estate};
+        for (DevBuf *b : ebufs) b->release();
         for (cudaEvent_t e : s.timer.ev) cudaEventDestroy(e);
     }
     delete h;
@@ -793,6 +931,23 @@ int gppd_centres(gppd_handle h, int slot, int64_t ntables, double *centres) {
     CK(cudaStreamSynchronize(s.stream));
     CK(cudaMemcpy(centres, s.centres.p, sizeof(double2) * NCHAN * (size_t)ntables,
                   cudaMemcpyDeviceToHost));
+    return GPPD_OK;
+}
+
+int gppd_ellipses(gppd_handle h, int slot, int64_t ntables, double *ell, int32_t *status) {
+    int rc = check_handle(h);
+    if (rc) return rc;
+    if (slot < 0 || slot >= NSLOTS || !ell || ntables < 1) return GPPD_ERR_ARG;
+    Slot &s = h->slots[slot];
+    if (ntables > s.nellipses) {
+        g_last_error = "ellipses: the last call on this slot fitted fewer tables' ellipses";
+        return GPPD_ERR_ARG;
+    }
+    CK(cudaStreamSynchronize(s.stream));
+    CK(cudaMemcpy(ell, s.ell.p, sizeof(double) * GPPD_ELLIPSE_STRIDE * NCHAN * (size_t)ntables,
+                  cudaMemcpyDeviceToHost));
+    if (status)
+        CK(cudaMemcpy(status, s.estatus.p, sizeof(int32_t) * NCHAN * (size_t)ntables, cudaMemcpyDeviceToHost));
     return GPPD_OK;
 }
 
@@ -934,6 +1089,10 @@ int gppd_demodulate_f64(gppd_handle h, int64_t n, int64_t nwindow, const double 
         g_last_error = "demodulate_f64: null buffer or n < 2";
         return GPPD_ERR_ARG;
     }
+    if (opt && (opt->flags & GPPD_CENTER_ELLIPSE)) {
+        g_last_error = "GPPD_CENTER_ELLIPSE applies to the table entry points only";
+        return GPPD_ERR_UNSUPPORTED;
+    }
     Slot &s = h->slots[0];
     cudaStream_t st = s.stream;
     CK(cudaStreamSynchronize(st));
@@ -995,6 +1154,10 @@ int gppd_demodulate_f64_dev(gppd_handle h, int slot, void *stream, int64_t n, in
     if (slot < 0 || slot >= NSLOTS || !d_t || !d_data || !d_out || !d_params || !d_chi2 || n < 2) {
         g_last_error = "demodulate_f64_dev: bad slot, null buffer or n < 2";
         return GPPD_ERR_ARG;
+    }
+    if (opt && (opt->flags & GPPD_CENTER_ELLIPSE)) {
+        g_last_error = "GPPD_CENTER_ELLIPSE applies to the table entry points only";
+        return GPPD_ERR_UNSUPPORTED;
     }
     Slot &s = h->slots[slot];
     cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
@@ -1093,7 +1256,7 @@ int gppd_submit_table_f32(gppd_handle h, int slot, int64_t n, const int32_t *tim
     a.d_chi2 = s.chi2.as<double>();
     a.d_info = s.info.as<int>();
     a.d_state_out = s.state_out.as<int8_t>();
-    if ((rc = run_batch(h, s, st, tabs, &o, nullptr, false))) return rc;
+    if ((rc = run_tables(h, s, st, tabs, o))) return rc;
     CK(cudaMemcpyAsync(volt_out, s.volt_out.p, obytes, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(params, s.params.p, sizeof(double) * 6 * nfits, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(chi2, s.chi2.p, sizeof(double) * nfits, cudaMemcpyDeviceToHost, st));
@@ -1173,7 +1336,7 @@ static int submit_rows_core(gppd_handle h, int slot, int64_t n, const void *rows
     a.d_chi2 = s.chi2.as<double>();
     a.d_info = s.info.as<int>();
     a.d_state_out = s.state_out.as<int8_t>();
-    if ((rc = run_batch(h, s, st, tabs, &o, nullptr, false))) return rc;
+    if ((rc = run_tables(h, s, st, tabs, o))) return rc;
     launch_pack_rows(L, s.rows.p, n, row_bytes, volt_off, s.volt_out.as<float>(), out_floats, s.rows_out.p,
                      row_bytes_out);
     CK(cudaGetLastError());
@@ -1596,6 +1759,7 @@ int gppd_process_tables_f32_dev(gppd_handle h, int slot, void *stream, int64_t n
     }
     // FAINT tables and bright tables as two concurrent chains (results do not depend
     // on the batching: all partial sums are over fixed row segments)
+    if (o.flags & GPPD_CENTER_ELLIPSE) return run_batch_ellipse(h, s, st, tabs, o);
     std::vector<TableArgs> faint, bright;
     for (TableArgs &a : tabs) (a.n1 > 0 ? faint : bright).push_back(a);
     // (the fit's latency-bound tail and the HBM-bound demodulation of one chain overlap the

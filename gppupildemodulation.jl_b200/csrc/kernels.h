@@ -42,6 +42,22 @@ int circle_max_segments(long long max_rows);
 void launch_circle(const Launcher &L, const TableDesc *d_tabs, int ntables, long long max_rows,
                    double *d_part);
 
+// `--center ellipse` (GPPD_CENTER_ELLIPSE, centre_kernels.cu).  On kind-0 descriptors whose
+// tv.t / tv.data point at the corrected arrays and ov.out at the demodulated ones:
+//   launch_ellipse_fit    the ten circle sums + five fourth-order ones over the same fixed
+//                         segments (d_part: [ntables][circle_max_segments][ELL_VALS][40]),
+//                         then one conic per channel -> d_ell [ntables][40][ELL_STRIDE]
+//                         = (x0, y0, r, alpha, m21, m22), d_status [ntables][40]
+//   launch_ellipse_apply  TIME + VOLT rows -> t [n] f64 and corrected data [40][n] complex128
+//   launch_repack_arrays  demodulated out [40][n] complex128 -> float32 VOLT rows of ov
+constexpr int ELL_VALS = 15;
+constexpr int ELL_STRIDE = 6;
+void launch_ellipse_fit(const Launcher &L, const TableDesc *d_tabs, int ntables, long long max_rows,
+                        double *d_part, double *d_ell, int *d_status);
+void launch_ellipse_apply(const Launcher &L, const TableDesc *d_tabs, int ntables, long long max_rows,
+                          const double *d_ell);
+void launch_repack_arrays(const Launcher &L, const TableDesc *d_tabs, int ntables, long long max_rows, bool keepraw);
+
 // Jacobi-Anger harmonic sums of every fit + reduction into the harmonic table
 int harm_max_segments(long long max_rows_per_job);   // fixed 6144-row segments
 int stats_max_segments(long long max_rows_per_job);  // fixed 1024-row segments

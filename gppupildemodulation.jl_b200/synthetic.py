@@ -60,13 +60,19 @@ def faint_header(mjd: float, t_first: float = 10.0, rate: float = 3.0,
 
 def make_table(nrows: int = 100_000, k: int = 0, faint: bool = False,
                jitter: bool = False, noise: float = 0.02, centred: bool = False,
-               state=None, seed: int | None = None):
+               state=None, seed: int | None = None, quadrature=None):
     """One synthetic file.  Returns a dict with
     ``time_us`` (N,) int32, ``volt`` (N,80) float32, ``mjd``, ``truth``
     (dict of the generating a, b, phi, c per diode), ``header`` (keywords).
     ``state``: optional int8 MetState vector used for the power scale in FAINT
     files (NORMAL 1.0 / HIGH 3.0 / LOW 0.2 / others 1.0); callers obtain it
-    from ``buildstates`` so that generator and segmentation agree."""
+    from ``buildstates`` so that generator and segmentation agree.
+    ``quadrature``: imperfect quadrature detectors (``--center ellipse``), ``(r[40],
+    alpha[40])`` or ``True`` for r ~ U(0.85, 1.15), alpha ~ U(-0.15, 0.15) rad drawn from
+    a generator of their own (the other draws, hence the default output, do not change).
+    Each channel is distorted about its generating centre c with the Heydemann forward
+    model x = c.re + U1, y = c.im + (U2 cos alpha - U1 sin alpha) / r; ``truth`` then holds
+    ``quad_r``, ``quad_alpha`` and the 40 generating centres ``centres``."""
     mjd = 59949.0 + k / 100.0
     rng = np.random.Generator(np.random.PCG64(20230105 + k if seed is None else seed))
     time_us = (2000 * np.arange(nrows, dtype=np.int64))
@@ -84,12 +90,28 @@ def make_table(nrows: int = 100_000, k: int = 0, faint: bool = False,
         st = np.asarray(state)
         pscale = np.where(st == 3, 3.0, np.where(st == 1, 0.2, 1.0))
     wt = M_2PI * t
+    quad = None
+    if quadrature is True:
+        qrng = np.random.Generator(np.random.PCG64(77_000_000 + (k if seed is None else seed)))
+        quad = (qrng.uniform(0.85, 1.15, size=40), qrng.uniform(-0.15, 0.15, size=40))
+    elif quadrature is not None:
+        quad = (np.asarray(quadrature[0], dtype=np.float64).reshape(40),
+                np.asarray(quadrature[1], dtype=np.float64).reshape(40))
+    gen_c = np.zeros(40, dtype=np.complex128) if centred else centres
+
+    def distort(z, ch):
+        if quad is None:
+            return z
+        r, al = quad[0][ch], quad[1][ch]
+        u = z - gen_c[ch]
+        return gen_c[ch] + (u.real + 1j * ((u.imag * np.cos(al) - u.real * np.sin(al)) / r))
+
     for side in (0, 16):
         for tel in range(1, 5):
             fc_ch = 32 + side // 4 + (tel - 1)
             phi_fc = np.cumsum(rng.normal(0.0, 0.02, size=nrows)) + rng.uniform(-np.pi, np.pi)
             fc = (0.0 if centred else centres[fc_ch]) + 0.3 * np.exp(1j * phi_fc)
-            fc = fc + 0.002 * (rng.normal(size=nrows) + 1j * rng.normal(size=nrows))
+            fc = distort(fc + 0.002 * (rng.normal(size=nrows) + 1j * rng.normal(size=nrows)), fc_ch)
             volt[:, 2 * fc_ch] = fc.real
             volt[:, 2 * fc_ch + 1] = fc.imag
             for dio in range(4):
@@ -100,10 +122,12 @@ def make_table(nrows: int = 100_000, k: int = 0, faint: bool = False,
                 phi = rng.uniform(-np.pi, np.pi)
                 c = 0.0 if centred else centres[ch]
                 e = noise * amp * (rng.normal(size=nrows) + 1j * rng.normal(size=nrows))
-                d = c + a * pscale * np.exp(1j * phi_fc) * np.exp(1j * b * np.sin(wt + phi)) + e
+                d = distort(c + a * pscale * np.exp(1j * phi_fc) * np.exp(1j * b * np.sin(wt + phi)) + e, ch)
                 volt[:, 2 * ch] = d.real
                 volt[:, 2 * ch + 1] = d.imag
                 truth["a"][ch], truth["b"][ch], truth["phi"][ch], truth["c"][ch] = a, b, phi, c
+    if quad is not None:
+        truth["quad_r"], truth["quad_alpha"], truth["centres"] = quad[0], quad[1], gen_c.copy()
     header = faint_header(mjd) if faint else {
         "MJD-OBS": mjd, "ESO INS MET MODE": "ON", "ESO INS PMC1 MODULATE": True}
     return dict(time_us=time_us, volt=volt, mjd=mjd, truth=truth, header=header)

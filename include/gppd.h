@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define GPPD_VERSION 122 /* 0.1.22: + GPPD_FP32; 0.1.21: + gppd_file_* (native ingest); 0.1.20: gppd_options.group_mask, gppd_demodulate_f64_dev (0.1.10: gppd_submit_fits_rows,
+#define GPPD_VERSION 122 /* 0.1.22: + GPPD_FP32, GPPD_CENTER_ELLIPSE / gppd_ellipses; 0.1.21: + gppd_file_* (native ingest); 0.1.20: gppd_options.group_mask, gppd_demodulate_f64_dev (0.1.10: gppd_submit_fits_rows,
                             gppd_centres, gppd_set_split_chains, gppd_debug_harmonics, GPPD_CENTER_EMPIRICAL) */
 
 /* ---- status codes ------------------------------------------------------ */
@@ -56,6 +56,36 @@ extern "C" {
                                points only; their `offsets` argument is then ignored and
                                GPPD_FITOFFSETS is off.  (The reference itself throws on
                                this path: its `Circle` type is undefined.) */
+#define GPPD_CENTER_ELLIPSE 0x80u /* (= 128) `--center ellipse`: offset AND ellipse
+                               (Heydemann) correction of each of the 40 channels, for quadrature detectors whose two outputs
+                               differ in gain (ratio r) or are not exactly in quadrature (error
+                               alpha).  Per channel, over the samples compute_offsets uses (all
+                               rows, or the HIGH rows of a FAINT table): the algebraic
+                               least-squares conic A u^2 + B uv + C v^2 + D u + E v + F = 0 with
+                               A + C = 1 (solved on samples shifted to their centroid and scaled
+                               to unit rms radius); centre [2A B; B 2C] (x0, y0) = -(D, E),
+                               r = sqrt(C/A), alpha = asin(B / (2 sqrt(AC))), i.e. the forward
+                               model x = x0 + U1, y = y0 + (U2 cos alpha - U1 sin alpha) / r.
+                               Every row, in every state, is then corrected in float64 with
+                               every operation rounded (no FMA):
+                                   m21 = tan alpha, m22 = r / cos alpha
+                                   x' = x - x0,  y' = m21 x' + m22 (y - y0)
+                               (the x-axis scale is kept: |a| stays in volts of the x output),
+                               and the corrected channels replace the centred ones everywhere
+                               downstream (NoOffsets fit, FC phasor, FAINT statistics, output
+                               VOLT including the FC columns; keepraw: columns 1..80 stay raw).
+                               A channel falls back to the empirical circle centre and the
+                               identity shape (status 1) when it has fewer than 5 samples, the
+                               Cholesky factorisation of the 5x5 normal matrix meets a pivot
+                               <= 1e-12 of its diagonal entry, A <= 0 or C <= 0, or the axis
+                               ratio exceeds 10 (4AC - B^2 <= 4 * 0.01 / 1.01^2); with no circle
+                               either, to centre 0 and the identity (status 0).  Table entry
+                               points only (gppd_demodulate_f64* return GPPD_ERR_UNSUPPORTED);
+                               their `offsets` argument is ignored; with GPPD_FITOFFSETS or
+                               GPPD_CENTER_EMPIRICAL the call fails with GPPD_ERR_ARG.
+                               GPPD_FP32 has no effect in this mode (the array path the
+                               corrected channels take has no FP32 form).  gppd_ellipses
+                               returns the fitted maps. */
 
 #define GPPD_FP32 64u /* OPTIONAL reduced precision, off by default: the harmonic sums of the fit are
                          formed from float32 stream values and harmonics rounded to 23-bit fixed
@@ -323,6 +353,15 @@ int gppd_process_tables_f32_dev(gppd_handle h, int slot, void *stream, int64_t n
 int gppd_centres(gppd_handle h, int slot, int64_t ntables, double *centres);
 
 /*
+ * The maps the last GPPD_CENTER_ELLIPSE call on pipeline slot `slot` fitted and applied:
+ * ell [ntables][40][GPPD_ELLIPSE_STRIDE] = (x0, y0, r, alpha, m21, m22) and, unless NULL,
+ * status [ntables][40] = 2 (ellipse), 1 (no ellipse: circle centre, identity shape) or
+ * 0 (no circle either: centre 0, identity).  Waits like gppd_centres.
+ */
+#define GPPD_ELLIPSE_STRIDE 6
+int gppd_ellipses(gppd_handle h, int slot, int64_t ntables, double *ell, int32_t *status);
+
+/*
  * Test hook: the harmonic-sum table of the last batch of pipeline slot `slot`
  * (value-major, [value][fit]; see csrc/gppd_device.cuh), so that the tests can hold the
  * two implementations of the sums (FP64 DMMA, int8 tensor cores) against each other.
@@ -349,10 +388,11 @@ int64_t gppd_launch_count(gppd_handle h);
  * of the launch sequence).  ms[p] / counts[p] accumulate over all slots since
  * the last reset; gppd_pass_times waits for the recorded events. */
 #define GPPD_PASS_SEGMENT 0 /* FAINT segmentation (buildstates)          */
-#define GPPD_PASS_BASIS 1   /* per-row sin/cos basis + job ranges         */
+#define GPPD_PASS_BASIS 1   /* per-row sin/cos basis + job ranges (+ the centre fits and the
+                               ellipse correction of --center empirical / ellipse) */
 #define GPPD_PASS_STATS 2   /* per-state mean/variance (FAINT)            */
 #define GPPD_PASS_FIT 3     /* the modulation fit (NEWUOA + objective)    */
-#define GPPD_PASS_DEMOD 4   /* demodulation + repack                      */
+#define GPPD_PASS_DEMOD 4   /* demodulation + repack (+ the ellipse mode's repack) */
 #define GPPD_PASS_EXPORT 5  /* parameter export                           */
 #define GPPD_PASS_HARMONICS 6 /* Jacobi-Anger harmonic sums (harmonic evaluator) */
 #define GPPD_PASS_FALLBACK 7  /* direct re-fit of the fits the harmonic evaluator gave up on */

@@ -35,6 +35,8 @@ const GPPD_NO_RECENTER = UInt32(4)
 const GPPD_KEEPRAW     = UInt32(8)
 const GPPD_CENTER_EMPIRICAL = UInt32(32)
 const GPPD_FP32        = UInt32(64)   # optional reduced-precision harmonic sums (off by default)
+const GPPD_CENTER_ELLIPSE = UInt32(128)   # `--center ellipse`: offset + ellipse correction per channel
+const GPPD_ELLIPSE_STRIDE = 6
 
 # struct gppd_options (include/gppd.h)
 struct Options
@@ -141,18 +143,22 @@ work of `processmetrology` (src/GPPupilDemodulation.jl:139-171,192-253) and the 
 decoding of `Dict(hdu)` (src/FitsUtils.jl:31-37).  `rows_out` receives the output records
 (`row_bytes + 256` bytes each with `keepraw`).  `offsets === nothing` fits the centres;
 `offsets === true` (processmetrology's default, `--center empirical`) has the library fit
-one circle per channel (compute_offsets, :105-125) -- `centres(slot)` returns them.
+one circle per channel (compute_offsets, :105-125) -- `centres(slot)` returns them;
+`offsets === :ellipse` (`--center ellipse`) one ellipse per channel, applied to every row
+before the fit -- `ellipses(slot)` returns the maps.
 """
 function processrows!(rows_out::Vector{UInt8}, rows::Vector{UInt8}, row_bytes::Integer,
                       time_off::Integer, volt_off::Integer, mjd::Real;
-                      offsets::Union{Nothing,Bool,Vector{ComplexF64}} = nothing,
+                      offsets::Union{Nothing,Bool,Symbol,Vector{ComplexF64}} = nothing,
                       faintparam::Union{Nothing,FaintStates} = nothing,
                       window::Real = 0.0, keepraw::Bool = false, onlyhigh::Bool = false, slot::Integer = 0,
                       fp32::Bool = false)
     n = length(rows) ÷ row_bytes
     flags = (onlyhigh ? GPPD_ONLYHIGH : UInt32(0)) | (keepraw ? GPPD_KEEPRAW : UInt32(0)) |
-            (offsets === true ? GPPD_CENTER_EMPIRICAL : UInt32(0)) | (fp32 ? GPPD_FP32 : UInt32(0))
-    offsets isa Bool && (offsets = nothing)
+            (offsets === true ? GPPD_CENTER_EMPIRICAL : UInt32(0)) | (fp32 ? GPPD_FP32 : UInt32(0)) |
+            (offsets === :ellipse ? GPPD_CENTER_ELLIPSE : UInt32(0))
+    offsets isa Symbol && offsets !== :ellipse && throw(ArgumentError("offsets: a vector, nothing, true or :ellipse"))
+    offsets isa Union{Bool,Symbol} && (offsets = nothing)
     opt = Options(flags, 0, 0, 0, (0.0, 0.0), 0.0, 0.0)
     nwrows = Ref{Int64}(0); nwin = Ref{Int64}(1)
     if window > 0
@@ -217,12 +223,14 @@ Queue one FITS file: `n` METROLOGY records of `row_bytes` bytes start at byte `d
 """
 function submitfile!(slot::Integer, path::AbstractString, data_offset::Integer, n::Integer,
                      row_bytes::Integer, time_off::Integer, volt_off::Integer, mjd::Real;
-                     offsets::Union{Nothing,Bool,Vector{ComplexF64}} = nothing,
+                     offsets::Union{Nothing,Bool,Symbol,Vector{ComplexF64}} = nothing,
                      faintparam::Union{Nothing,FaintStates} = nothing, window::Real = 0.0,
                      keepraw::Bool = false, onlyhigh::Bool = false)
     flags = (onlyhigh ? GPPD_ONLYHIGH : UInt32(0)) | (keepraw ? GPPD_KEEPRAW : UInt32(0)) |
-            (offsets === true ? GPPD_CENTER_EMPIRICAL : UInt32(0))
-    offsets isa Bool && (offsets = nothing)
+            (offsets === true ? GPPD_CENTER_EMPIRICAL : UInt32(0)) |
+            (offsets === :ellipse ? GPPD_CENTER_ELLIPSE : UInt32(0))
+    offsets isa Symbol && offsets !== :ellipse && throw(ArgumentError("offsets: a vector, nothing, true or :ellipse"))
+    offsets isa Union{Bool,Symbol} && (offsets = nothing)
     opt = Options(flags, 0, 0, 0, (0.0, 0.0), 0.0, 0.0)
     t1 = isnothing(faintparam) ? Float64[] : Vector{Float64}(faintparam.timer1)
     t2 = isnothing(faintparam) ? Float64[] : Vector{Float64}(faintparam.timer2)
@@ -283,6 +291,21 @@ function centres(slot::Integer = 0)
     gppd_assert_ok(ccall((:gppd_centres, libgppd), Cint, (Ptr{Cvoid}, Cint, Int64, Ptr{ComplexF64}),
                          gethandle(), slot, 1, c))
     return c
+end
+
+"""
+    ellipses(slot = 0) -> (ell, status)
+
+The maps fitted and applied by the last `offsets = :ellipse` call on `slot`: `ell` is a
+6 x 40 matrix, column c = (x0, y0, r, alpha, m21, m22) of channel c; `status[c]` is 2
+(ellipse), 1 (circle centre, identity shape) or 0 (neither).
+"""
+function ellipses(slot::Integer = 0)
+    ell = Matrix{Float64}(undef, GPPD_ELLIPSE_STRIDE, 40)
+    status = Vector{Int32}(undef, 40)
+    gppd_assert_ok(ccall((:gppd_ellipses, libgppd), Cint, (Ptr{Cvoid}, Cint, Int64, Ptr{Float64}, Ptr{Int32}),
+                         gethandle(), slot, 1, ell, status))
+    return ell, status
 end
 
 end # module

@@ -38,7 +38,7 @@ tgen = time.time() - t0
 res = {"workload": "night directory of %d FITS files x %d rows (30 %% FAINT), bin/GPPupilDemodulation -r" % (nfiles, rows),
        "base_directory": base, "input_gb": nfiles * rows * 332 / 1e9, "generation_seconds": tgen}
 env = dict(os.environ, GPPD_CLI_TIMING="1")
-for label, extra in (("native", []), ("python_records", ["--no-native"])):
+for label, extra in (("native", []), ("python_records", ["--no-native"]), ("ellipse", ["-c", "ellipse"])):
     runs, inner, detail = [], [], None
     for _ in range(3):                      # page cache / first-touch effects make single runs noisy
         shutil.rmtree(out, ignore_errors=True)
@@ -61,6 +61,7 @@ for label, extra in (("native", []), ("python_records", ["--no-native"])):
 res["note"] = ("command = wall clock of the whole command including interpreter start-up, library load and "
                "CUDA context creation; night = first file submitted to last file written, inside the process. "
                "native: records read / written by the library's I/O threads (gppd_file_*); python_records: "
-               "the same files through gppd_submit_fits_rows with Python reading and writing the records")
+               "the same files through gppd_submit_fits_rows with Python reading and writing the records; "
+               "ellipse: the native path with --center ellipse (offset + ellipse correction per channel)")
 print(json.dumps(res))
 shutil.rmtree(d, ignore_errors=True); shutil.rmtree(out, ignore_errors=True)
