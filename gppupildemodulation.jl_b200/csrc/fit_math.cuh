@@ -107,7 +107,9 @@ __device__ __forceinline__ double bessel_j_lane(double b, int lane) {
     return mine * (1.0 / (jc + 2.0 * seven));
 }
 
-// sin and cos of a moderate argument (|x| < 1e5), < 1 ulp: two-constant Cody-Waite
+// sin and cos of a moderate argument (|x| < 1e5), relative error below 2^-52 (at most 1.5 ulp,
+// where the reduced argument is near +-pi/4) and, near the zeros of sin and cos, absolute error
+// below 2^-52 |result| + 1e-28 (|k| |pi/2 - hi - lo| < 63 662 * 1.5e-33): two-constant Cody-Waite
 // reduction by pi/2 with FMAs (exact first step) and the fdlibm kernel polynomials in
 // Horner/FMA form.  About a third of the instructions of the general-purpose
 // sincos(), which carries a Payne-Hanek path.  Every operation is an explicit fma or
@@ -156,6 +158,36 @@ __device__ __forceinline__ void sincos_moderate(double x, double *sn, double *cs
     pc = fma(z, pc, -0.5);
     const double kc = fma(z, pc, 1.0);
     // quadrant: swap for odd k, then flip signs through the high words
+    const bool odd = k & 1;
+    const double s0 = odd ? kc : ks, c0 = odd ? ks : kc;
+    const int sflip = (k & 2) << 30, cflip = ((k + 1) & 2) << 30;
+    *sn = __hiloint2double(__double2hiint(s0) ^ sflip, __double2loint(s0));
+    *cs = __hiloint2double(__double2hiint(c0) ^ cflip, __double2loint(c0));
+}
+
+// sin and cos of the demodulation phase psi for the float32 table path: |error| < 2e-10,
+// i.e. 2^-32 -- the result is rounded to float32 (2^-24) right after, so a full-precision
+// double sincos would buy nothing.  psi = b sin(.) is a few radians at most: one-constant
+// Cody-Waite reduction by pi/2 (the quotient through the 1.5 * 2^52 rounding trick: no
+// conversion instruction, the XU pipe issues one warp instruction every 8 cycles) and the
+// leading terms of the fdlibm kernel polynomials.
+// The caller guarantees |x| < 1e4 (|psi| <= |b|: checked once per fit, not per row).
+__device__ __forceinline__ void sincos_demod(double x, double *sn, double *cs) {
+    const double t = fma(x, c_sincos[0], 6755399441055744.0);      // 1.5 * 2^52: low word = rint(x 2/pi)
+    const int k = __double2loint(t);
+    const double fn = t - 6755399441055744.0;
+    const double r = fma(-fn, c_sincos[1], x);                     // |fn| pi/2_lo < 1e-12
+    const double z = r * r;
+    double ps = fma(z, c_sincos[4], c_sincos[5]);                  // S5, S4
+    ps = fma(z, ps, c_sincos[6]);
+    ps = fma(z, ps, c_sincos[7]);
+    ps = fma(z, ps, c_sincos[8]);
+    const double ks = fma(z * r, ps, r);
+    double pc = fma(z, c_sincos[11], c_sincos[12]);                // C4, C3
+    pc = fma(z, pc, c_sincos[13]);
+    pc = fma(z, pc, c_sincos[14]);
+    pc = fma(z, pc, -0.5);
+    const double kc = fma(z, pc, 1.0);
     const bool odd = k & 1;
     const double s0 = odd ? kc : ks, c0 = odd ? ks : kc;
     const int sflip = (k & 2) << 30, cflip = ((k + 1) & 2) << 30;

@@ -803,7 +803,7 @@ __device__ __forceinline__ double2 demod_sample(const FitResult &fr, unsigned fl
         double gp = __dadd_rn(__dmul_rn(fr.b, sn), fr.alpha);
         double psi = __dadd_rn(gp, -fr.alpha);
         double sp, cp;
-        sincos_moderate(psi, &sp, &cp);      // < 1 ulp; falls back to sincos() beyond 1e5
+        sincos_moderate(psi, &sp, &cp);      // <= 1.5 ulp; falls back to sincos() beyond 1e5
         double vr = d.x, vi = d.y;
         if (flags & 2u) { vr -= fr.cre; vi -= fr.cim; }
         // (vr + j vi) * (cp - j sp)
@@ -822,36 +822,6 @@ __device__ __forceinline__ double2 demod_sample(const FitResult &fr, unsigned fl
     sincos(ang, &sa, &ca);
     return make_double2(__dadd_rn(__dmul_rn(d.x, ca), __dmul_rn(d.y, sa)),
                         __dadd_rn(__dmul_rn(d.y, ca), -__dmul_rn(d.x, sa)));
-}
-
-// sin and cos of the demodulation phase psi for the float32 table path: |error| < 2e-10,
-// i.e. 2^-32 -- the result is rounded to float32 (2^-24) right after, so a full-precision
-// double sincos would buy nothing.  psi = b sin(.) is a few radians at most: one-constant
-// Cody-Waite reduction by pi/2 (the quotient through the 1.5 * 2^52 rounding trick: no
-// conversion instruction, the XU pipe issues one warp instruction every 8 cycles) and the
-// leading terms of the fdlibm kernel polynomials.
-// The caller guarantees |x| < 1e4 (|psi| <= |b|: checked once per fit, not per row).
-__device__ __forceinline__ void sincos_demod(double x, double *sn, double *cs) {
-    const double t = fma(x, c_sincos[0], 6755399441055744.0);      // 1.5 * 2^52: low word = rint(x 2/pi)
-    const int k = __double2loint(t);
-    const double fn = t - 6755399441055744.0;
-    const double r = fma(-fn, c_sincos[1], x);                     // |fn| pi/2_lo < 1e-12
-    const double z = r * r;
-    double ps = fma(z, c_sincos[4], c_sincos[5]);                  // S5, S4
-    ps = fma(z, ps, c_sincos[6]);
-    ps = fma(z, ps, c_sincos[7]);
-    ps = fma(z, ps, c_sincos[8]);
-    const double ks = fma(z * r, ps, r);
-    double pc = fma(z, c_sincos[11], c_sincos[12]);                // C4, C3
-    pc = fma(z, pc, c_sincos[13]);
-    pc = fma(z, pc, c_sincos[14]);
-    pc = fma(z, pc, -0.5);
-    const double kc = fma(z, pc, 1.0);
-    const bool odd = k & 1;
-    const double s0 = odd ? kc : ks, c0 = odd ? ks : kc;
-    const int sflip = (k & 2) << 30, cflip = ((k + 1) & 2) << 30;
-    *sn = __hiloint2double(__double2hiint(s0) ^ sflip, __double2loint(s0));
-    *cs = __hiloint2double(__double2hiint(c0) ^ cflip, __double2loint(c0));
 }
 
 // METROLOGY tables (float32 rows).  Every WARP runs its own pipeline over a contiguous run of
@@ -912,7 +882,7 @@ __device__ __forceinline__ DemodK demod_constants(const FitResult *fr, bool offs
 // takes 4 x 32 rows of the block and loops over the channels.  When its rows belong to one job
 // with a uniform phase quantum (the usual case) the constants of a fit are loaded once per
 // channel and the four rows of a lane are independent chains; psi is a few radians, so the
-// < 1 ulp sincos_moderate replaces the general-purpose sincos (a third of its instructions).
+// sincos_moderate (<= 1.5 ulp) replaces the general-purpose sincos (a third of its instructions).
 // The other cases go sample by sample through demod_sample.
 __device__ __forceinline__ void demod_arrays_body(const TableDesc &tbg, const FitResult *results, unsigned flags) {
     const TableView &tv = tbg.tv;
