@@ -61,9 +61,17 @@ bool debug_sync() {
         }                                                                          \
     } while (0)
 
+// Buffers and events below free themselves: a Slot, a FileJob and the handle clean up by
+// destruction, so that no buffer has to be remembered in a list to be released.
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
     int ensure(size_t bytes) {
         if (bytes <= cap) return GPPD_OK;
         if (p) cudaFree(p);
@@ -78,11 +86,6 @@ struct DevBuf {
         }
         cap = want;
         return GPPD_OK;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
     }
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
@@ -99,12 +102,24 @@ struct PassTimer {
     std::vector<int> pass;            // pass id per pair
     double ms[NPASS] = {0};
     long long count[NPASS] = {0};
+    PassTimer() = default;
+    PassTimer(const PassTimer &) = delete;
+    PassTimer &operator=(const PassTimer &) = delete;
+    ~PassTimer() {
+        for (cudaEvent_t e : ev) cudaEventDestroy(e);
+    }
 };
 
 // page-locked host buffer owned by the library (native file ingest)
 struct PinBuf {
     void *p = nullptr;
     size_t cap = 0;
+    PinBuf() = default;
+    PinBuf(const PinBuf &) = delete;
+    PinBuf &operator=(const PinBuf &) = delete;
+    ~PinBuf() {
+        if (p) cudaFreeHost(p);
+    }
     int ensure(size_t bytes) {
         if (bytes <= cap) return GPPD_OK;
         if (p) cudaFreeHost(p);
@@ -118,11 +133,6 @@ struct PinBuf {
         }
         cap = want;
         return GPPD_OK;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
     }
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
@@ -308,8 +318,8 @@ struct PassScope {
 
 // One table of a batch, as the entry points describe it (device pointers).
 struct TableArgs {
-    TableView tv;
-    OutView ov;
+    TableView tv{};
+    OutView ov{};
     long long wrows = 0;            // <= 0 or >= n: whole table
     const int8_t *d_state_in = nullptr;
     const double *timer1 = nullptr, *timer2 = nullptr;  // HOST timers
@@ -394,15 +404,6 @@ int run_batch(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs
         return GPPD_ERR_ARG;
     }
     const bool direct = method == GPPD_METHOD_DIRECT;
-    const bool all_groups = ((fo.flags >> GROUP_MASK_SHIFT) & 0xffu) == 0xffu;
-    if (!all_groups && !segment_only) {
-        for (int t = 0; t < T; ++t) {
-            if (td[t].tv.kind != 1 || td[t].ov.kind != 1) {
-                g_last_error = "gppd_options.group_mask: a partial mask applies to the demodulate_f64 entry points only";
-                return GPPD_ERR_UNSUPPORTED;
-            }
-        }
-    }
     // the int8 tensor-core form of the harmonic sums takes dense METROLOGY tables (rows of
     // 80 floats, 16-byte aligned) and 16-byte aligned complex128 arrays; the other layouts
     // (strided FITS records before the unpack pass never get here) use the FP64 DMMA kernel.
@@ -635,21 +636,38 @@ int check_handle(gppd_handle h) {
     return GPPD_OK;
 }
 
+// The options of a table entry point: the caller's (or zeros) with the centre mode applied,
+// after the rejection of every combination that no table path runs.  The centre mode is the
 // offsets of processmetrology (src/GPPupilDemodulation.jl:150-157): a vector => subtract it;
 // true (GPPD_CENTER_EMPIRICAL) => circle centres fitted here; false (NULL) => fitoffsets.
-// GPPD_CENTER_ELLIPSE ignores the vector and keeps the caller's flags (run_batch_ellipse
-// refuses GPPD_FITOFFSETS and GPPD_CENTER_EMPIRICAL with it).
-void centre_mode(gppd_options &o, bool have_offsets) {
-    if (o.flags & GPPD_CENTER_ELLIPSE) return;
-    if (o.flags & GPPD_CENTER_EMPIRICAL) o.flags &= ~GPPD_FITOFFSETS;
-    else if (!have_offsets) o.flags |= GPPD_FITOFFSETS;
+// GPPD_CENTER_ELLIPSE ignores the vector.
+int table_options(const gppd_options *opt, bool have_offsets, gppd_options &o) {
+    memset(&o, 0, sizeof o);
+    if (opt) o = *opt;
+    if ((o.flags & GPPD_CENTER_ELLIPSE) && (o.flags & (GPPD_CENTER_EMPIRICAL | GPPD_FITOFFSETS))) {
+        g_last_error = "GPPD_CENTER_ELLIPSE excludes GPPD_CENTER_EMPIRICAL and GPPD_FITOFFSETS";
+        return GPPD_ERR_ARG;
+    }
+    if ((o.group_mask & 0xffu) != 0 && (o.group_mask & 0xffu) != 0xffu) {
+        g_last_error = "gppd_options.group_mask: a partial mask applies to the demodulate_f64 entry points only";
+        return GPPD_ERR_UNSUPPORTED;
+    }
+    if (!(o.flags & (GPPD_CENTER_EMPIRICAL | GPPD_CENTER_ELLIPSE)) && !have_offsets) o.flags |= GPPD_FITOFFSETS;
     else o.flags &= ~GPPD_FITOFFSETS;
+    return GPPD_OK;
+}
+
+// The options of the array entry points: GPPD_CENTER_ELLIPSE corrects METROLOGY tables only.
+int check_array_options(const gppd_options *opt) {
+    if (opt && (opt->flags & GPPD_CENTER_ELLIPSE)) {
+        g_last_error = "GPPD_CENTER_ELLIPSE applies to the table entry points only";
+        return GPPD_ERR_UNSUPPORTED;
+    }
+    return GPPD_OK;
 }
 
 void table_views(int64_t n, double mjd, const int32_t *d_time, const float *d_volt,
                  const double *d_offsets, float *d_volt_out, uint32_t flags, TableArgs &a) {
-    memset(&a.tv, 0, sizeof a.tv);
-    memset(&a.ov, 0, sizeof a.ov);
     a.tv.kind = 0;
     a.tv.big_endian = (flags & GPPD_BIG_ENDIAN) ? 1 : 0;
     a.tv.n = n;
@@ -666,6 +684,16 @@ void table_views(int64_t n, double mjd, const int32_t *d_time, const float *d_vo
     a.ov.volt_stride = a.ov.keepraw ? 576 : 320;
 }
 
+// the complex128-array counterpart (the demodulateall boundary): t[n], data[40][n] -> out[40][n]
+void array_views(int64_t n, const double *d_t, const double2 *d_data, double2 *d_out, TableArgs &a) {
+    a.tv.kind = 1;
+    a.tv.n = n;
+    a.tv.t = d_t;
+    a.tv.data = d_data;
+    a.ov.kind = 1;
+    a.ov.out = d_out;
+}
+
 // `--center ellipse` on a batch of kind-0 tables: a composition of existing passes around the
 // ellipse kernels (centre_kernels.cu), all on `stream`:
 //   1. FAINT segmentation of the tables that have timers (run_batch, segment_only)
@@ -675,14 +703,6 @@ void table_views(int64_t n, double mjd, const int32_t *d_time, const float *d_vo
 //   5. the repack of out into the caller's VOLT rows               (GPPD_PASS_DEMOD)
 int run_batch_ellipse(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs> &tabs,
                       const gppd_options &o) {
-    if (o.flags & (GPPD_CENTER_EMPIRICAL | GPPD_FITOFFSETS)) {
-        g_last_error = "GPPD_CENTER_ELLIPSE excludes GPPD_CENTER_EMPIRICAL and GPPD_FITOFFSETS";
-        return GPPD_ERR_ARG;
-    }
-    if ((o.group_mask & 0xffu) != 0 && (o.group_mask & 0xffu) != 0xffu) {
-        g_last_error = "gppd_options.group_mask: a partial mask applies to the demodulate_f64 entry points only";
-        return GPPD_ERR_UNSUPPORTED;
-    }
     const int T = (int)tabs.size();
     if (T <= 0) return GPPD_OK;
     long long R = 0, max_rows = 0, R_state = 0;
@@ -743,14 +763,7 @@ int run_batch_ellipse(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<T
             d.ov.out = s.eout.as<double2>() + NCHAN * row_off;
             d.state = states[t];
             TableArgs &b = arr[t];
-            memset(&b.tv, 0, sizeof b.tv);
-            memset(&b.ov, 0, sizeof b.ov);
-            b.tv.kind = 1;
-            b.tv.n = a.tv.n;
-            b.tv.t = d.tv.t;
-            b.tv.data = d.tv.data;
-            b.ov.kind = 1;
-            b.ov.out = d.ov.out;
+            array_views(a.tv.n, d.tv.t, d.tv.data, d.ov.out, b);
             b.wrows = a.wrows;
             b.d_state_in = states[t];
             b.d_params = a.d_params;
@@ -786,11 +799,139 @@ int run_batch_ellipse(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<T
     return GPPD_OK;
 }
 
-// the batch of a table entry point: the ellipse composition or the ordinary launch sequence
-int run_tables(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs> &tabs,
+// The batch of a table entry point on slot `slot`, with options from table_options: the ellipse
+// composition, the FAINT and the bright tables as two concurrent chains (the FAINT one on the
+// slot's aux stream), or one launch sequence.  Results do not depend on the batching: all
+// partial sums are over fixed row segments.
+int run_tables(gppd_handle h, int slot, cudaStream_t stream, std::vector<TableArgs> &tabs,
                const gppd_options &o) {
+    Slot &s = h->slots[slot];
     if (o.flags & GPPD_CENTER_ELLIPSE) return run_batch_ellipse(h, s, stream, tabs, o);
-    return run_batch(h, s, stream, tabs, &o, nullptr, false);
+    std::vector<TableArgs> faint, bright;
+    for (TableArgs &a : tabs) (a.n1 > 0 ? faint : bright).push_back(a);
+    // (the fit's latency-bound tail and the HBM-bound demodulation of one chain overlap the
+    // issue-bound harmonic pass of the other: measured +8 % on the 100-table night.  Each
+    // pass is then two launches per batch; gppd_pass_times adds their durations.
+    // GPPD_SPLIT_CHAINS=0 or gppd_set_split_chains(h, 0) keeps one launch sequence.)
+    // (not for batches of very many small fits: there the one-thread-per-fit solver dominates
+    // and two concurrent launches of it are slower than one -- measured, 20 tables: 5 000-row
+    // windows (12 800 fits) 3.3 against 4.3 ms, 2 000-row windows (32 000 fits) 5.0 against 4.3)
+    long long nfits_total = 0;
+    for (const TableArgs &a : tabs) {
+        const long long w = (a.wrows <= 0 || a.wrows >= a.tv.n) ? a.tv.n : a.wrows;
+        nfits_total += (a.tv.n + w - 1) / w * NDIODE;
+    }
+    if (faint.empty() || bright.empty() || !h->split_chains || nfits_total > 16384 ||
+        (o.flags & GPPD_CENTER_EMPIRICAL))
+        return run_batch(h, s, stream, tabs, &o, nullptr, false);
+    Slot &sb = h->aux[slot];
+    int rc;
+    CK(cudaEventRecord(sb.fork, stream));
+    CK(cudaStreamWaitEvent(sb.stream, sb.fork, 0));
+    if ((rc = run_batch(h, sb, sb.stream, faint, &o, nullptr, false))) return rc;
+    if ((rc = run_batch(h, s, stream, bright, &o, nullptr, false))) return rc;
+    CK(cudaEventRecord(sb.join, sb.stream));
+    CK(cudaStreamWaitEvent(stream, sb.join, 0));
+    return GPPD_OK;
+}
+
+// Rows per window and number of windows of a table of FITS records: gppd_table_windows on the
+// TIME of the first two records, read big-endian on the host (src/GPPupilDemodulation.jl:192),
+// once TIME and VOLT are known to lie inside the record without overlapping.
+int record_windows(int64_t n, const unsigned char *rows, int64_t row_bytes, int64_t time_off, int64_t volt_off,
+                   double mjd, double window_s, int64_t &wrows, int64_t &nwin) {
+    if (time_off < 0 || volt_off < 0 || time_off + 4 > row_bytes || volt_off + 320 > row_bytes ||
+        (time_off + 4 > volt_off && time_off < volt_off + 320)) {
+        g_last_error = "fits rows: TIME or VOLT outside the record";
+        return GPPD_ERR_ARG;
+    }
+    int32_t t01[2];
+    for (int k = 0; k < 2; ++k) {
+        const unsigned char *p = rows + k * row_bytes + time_off;
+        t01[k] = (int32_t)(((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | p[3]);
+    }
+    return gppd_table_windows(n, t01, mjd, window_s, &wrows, &nwin);
+}
+
+// One table of a host-buffer entry point, enqueued on the stream of slot `slot`.  The table is
+// either TIME + VOLT arrays (`rows` null) or FITS records (`rows`: big-endian, `row_bytes`
+// apart, TIME at `time_off` and VOLT at `volt_off`; already in s.rows when `rows_uploaded`).
+// `out` receives VOLT rows in the form of the input: arrays, or records with VOLT replaced.
+int stage_table(gppd_handle h, int slot, int64_t n, const int32_t *time_us, const float *volt, const void *rows,
+                bool rows_uploaded, int64_t row_bytes, int64_t time_off, int64_t volt_off, double mjd,
+                const double *offsets, const double *timer1, int64_t n1, const double *timer2, int64_t n2,
+                double window_s, const gppd_options *opt, void *out, double *params, double *chi2,
+                int32_t *info, int8_t *state_out) {
+    const bool recs = rows != nullptr;
+    int64_t wrows = n, nwin = 1;
+    int rc = recs ? record_windows(n, reinterpret_cast<const unsigned char *>(rows), row_bytes, time_off,
+                                   volt_off, mjd, window_s, wrows, nwin)
+                  : gppd_table_windows(n, time_us, mjd, window_s, &wrows, &nwin);
+    if (rc) return rc;
+    gppd_options o;
+    if ((rc = table_options(opt, offsets != nullptr, o))) return rc;
+    if (recs) o.flags &= ~GPPD_BIG_ENDIAN;    // the unpack pass delivers little-endian arrays
+    const int out_floats = (o.flags & GPPD_KEEPRAW) ? 144 : 80;
+    const int64_t row_bytes_out = row_bytes + 4 * (out_floats - 80);
+    const size_t nfits = (size_t)nwin * NDIODE;
+    const size_t vbytes = sizeof(float) * 80 * (size_t)n, obytes = sizeof(float) * out_floats * (size_t)n;
+    Slot &s = h->slots[slot];
+    cudaStream_t st = s.stream;
+    if (!rows_uploaded) CK(cudaStreamSynchronize(st));  // slot reuse: previous table of this slot must be done
+    std::lock_guard<std::mutex> lk(h->launch_mutex);
+    if (recs) {
+        if ((rc = s.rows.ensure((size_t)n * (size_t)row_bytes))) return rc;
+        if ((rc = s.rows_out.ensure((size_t)n * (size_t)row_bytes_out))) return rc;
+    }
+    if ((rc = s.time.ensure(sizeof(int32_t) * (size_t)n))) return rc;
+    if ((rc = s.volt.ensure(vbytes))) return rc;
+    if ((rc = s.volt_out.ensure(obytes))) return rc;
+    if ((rc = s.params.ensure(sizeof(double) * 6 * nfits))) return rc;
+    if ((rc = s.chi2.ensure(sizeof(double) * nfits))) return rc;
+    if ((rc = s.info.ensure(sizeof(int) * GPPD_INFO_STRIDE * nfits))) return rc;
+    if ((rc = s.state_out.ensure((size_t)n))) return rc;
+    if ((rc = s.offsets.ensure(sizeof(double) * 80))) return rc;
+    if (!recs) {
+        CK(cudaMemcpyAsync(s.time.p, time_us, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(s.volt.p, volt, vbytes, cudaMemcpyHostToDevice, st));
+    } else if (!rows_uploaded) {
+        CK(cudaMemcpyAsync(s.rows.p, rows, (size_t)n * (size_t)row_bytes, cudaMemcpyHostToDevice, st));
+    }
+    if (offsets)
+        CK(cudaMemcpyAsync(s.offsets.p, offsets, sizeof(double) * 80, cudaMemcpyHostToDevice, st));
+    Launcher L{st, &h->launches};
+    if (recs)
+        launch_unpack_rows(L, s.rows.p, n, row_bytes, time_off, volt_off, s.time.as<int32_t>(), s.volt.as<float>());
+    std::vector<TableArgs> tabs(1);
+    TableArgs &a = tabs[0];
+    table_views(n, mjd, s.time.as<int32_t>(), s.volt.as<float>(),
+                offsets ? s.offsets.as<double>() : nullptr, s.volt_out.as<float>(), o.flags, a);
+    a.wrows = wrows;
+    const bool faint = timer1 && timer2 && n1 > 0 && n2 > 0;
+    a.timer1 = timer1;
+    a.timer2 = timer2;
+    a.n1 = faint ? n1 : 0;
+    a.n2 = faint ? n2 : 0;
+    a.d_params = s.params.as<double>();
+    a.d_chi2 = s.chi2.as<double>();
+    a.d_info = s.info.as<int>();
+    a.d_state_out = s.state_out.as<int8_t>();
+    if ((rc = run_tables(h, slot, st, tabs, o))) return rc;
+    if (recs) {
+        launch_pack_rows(L, s.rows.p, n, row_bytes, volt_off, s.volt_out.as<float>(), out_floats, s.rows_out.p,
+                         row_bytes_out);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(out, s.rows_out.p, (size_t)n * (size_t)row_bytes_out, cudaMemcpyDeviceToHost, st));
+    } else {
+        CK(cudaMemcpyAsync(out, s.volt_out.p, obytes, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaMemcpyAsync(params, s.params.p, sizeof(double) * 6 * nfits, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(chi2, s.chi2.p, sizeof(double) * nfits, cudaMemcpyDeviceToHost, st));
+    if (info)
+        CK(cudaMemcpyAsync(info, s.info.p, sizeof(int) * GPPD_INFO_STRIDE * nfits, cudaMemcpyDeviceToHost, st));
+    if (state_out && faint)
+        CK(cudaMemcpyAsync(state_out, s.state_out.p, (size_t)n, cudaMemcpyDeviceToHost, st));
+    return GPPD_OK;
 }
 
 }  // namespace
@@ -862,7 +1003,7 @@ int gppd_create(int device, gppd_handle *out) {
         if (es == cudaSuccess) es = cudaEventCreateWithFlags(&h->aux[i].join, cudaEventDisableTiming);
         if (es != cudaSuccess) {
             g_last_error = cudaGetErrorString(es);
-            delete h;
+            gppd_destroy(h);
             return GPPD_ERR_CUDA;
         }
     }
@@ -874,11 +1015,6 @@ int gppd_destroy(gppd_handle h) {
     if (!h) return GPPD_OK;
     cudaSetDevice(h->device);
     gppd_file_drain(h);
-    for (int i = 0; i < NSLOTS; ++i) {
-        FileJob &f = h->slots[i].file;
-        PinBuf *pins[] = {&f.rows, &f.rows_out, &f.params, &f.chi2, &f.info, &f.state};
-        for (PinBuf *b : pins) b->release();
-    }
     for (int i = 0; i < 2 * NSLOTS; ++i) {
         Slot &s = i < NSLOTS ? h->slots[i] : h->aux[i - NSLOTS];
         if (s.stream) {
@@ -887,18 +1023,8 @@ int gppd_destroy(gppd_handle h) {
         }
         if (s.fork) cudaEventDestroy(s.fork);
         if (s.join) cudaEventDestroy(s.join);
-        DevBuf *bufs[] = {&s.rows, &s.rows_out, &s.time, &s.volt, &s.volt_out, &s.t, &s.data, &s.out, &s.state_in,
-                          &s.offsets, &s.params, &s.chi2, &s.info, &s.trace, &s.state_out,
-                          &s.state, &s.basis, &s.z, &s.y, &s.thkeys, &s.nvalid, &s.jobs,
-                          &s.results, &s.spart1, &s.spart2, &s.partZ, &s.partY, &s.htab,
-                          &s.timers, &s.lb, &s.events, &s.flags, &s.tabs, &s.exps, &s.faintjobs, &s.fbq,
-                          &s.centres, &s.cpart};
-        for (DevBuf *b : bufs) b->release();
-        DevBuf *ebufs[] = {&s.etabs, &s.ell, &s.estatus, &s.epart, &s.et, &s.edata, &s.eout, &s.estate};
-        for (DevBuf *b : ebufs) b->release();
-        for (cudaEvent_t e : s.timer.ev) cudaEventDestroy(e);
     }
-    delete h;
+    delete h;   // (the slots' buffers and pass timers free themselves, on the handle's device)
     return GPPD_OK;
 }
 
@@ -1059,11 +1185,7 @@ int gppd_buildstates(gppd_handle h, int64_t n, const double *t, const double *ti
     CK(cudaMemcpyAsync(s.t.p, t, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st));
     std::vector<TableArgs> tabs(1);
     TableArgs &a = tabs[0];
-    memset(&a.tv, 0, sizeof a.tv);
-    memset(&a.ov, 0, sizeof a.ov);
-    a.tv.kind = 1;
-    a.tv.n = n;
-    a.tv.t = s.t.as<double>();
+    array_views(n, s.t.as<double>(), nullptr, nullptr, a);
     a.timer1 = timer1;
     a.timer2 = timer2;
     a.n1 = n1;
@@ -1089,10 +1211,7 @@ int gppd_demodulate_f64(gppd_handle h, int64_t n, int64_t nwindow, const double 
         g_last_error = "demodulate_f64: null buffer or n < 2";
         return GPPD_ERR_ARG;
     }
-    if (opt && (opt->flags & GPPD_CENTER_ELLIPSE)) {
-        g_last_error = "GPPD_CENTER_ELLIPSE applies to the table entry points only";
-        return GPPD_ERR_UNSUPPORTED;
-    }
+    if ((rc = check_array_options(opt))) return rc;
     Slot &s = h->slots[0];
     cudaStream_t st = s.stream;
     CK(cudaStreamSynchronize(st));
@@ -1116,14 +1235,7 @@ int gppd_demodulate_f64(gppd_handle h, int64_t n, int64_t nwindow, const double 
 
     std::vector<TableArgs> tabs(1);
     TableArgs &a = tabs[0];
-    memset(&a.tv, 0, sizeof a.tv);
-    memset(&a.ov, 0, sizeof a.ov);
-    a.tv.kind = 1;
-    a.tv.n = n;
-    a.tv.t = s.t.as<double>();
-    a.tv.data = s.data.as<double2>();
-    a.ov.kind = 1;
-    a.ov.out = s.out.as<double2>();
+    array_views(n, s.t.as<double>(), s.data.as<double2>(), s.out.as<double2>(), a);
     a.wrows = nwindow;
     a.d_state_in = state ? s.state_in.as<int8_t>() : nullptr;
     a.d_params = s.params.as<double>();
@@ -1155,22 +1267,12 @@ int gppd_demodulate_f64_dev(gppd_handle h, int slot, void *stream, int64_t n, in
         g_last_error = "demodulate_f64_dev: bad slot, null buffer or n < 2";
         return GPPD_ERR_ARG;
     }
-    if (opt && (opt->flags & GPPD_CENTER_ELLIPSE)) {
-        g_last_error = "GPPD_CENTER_ELLIPSE applies to the table entry points only";
-        return GPPD_ERR_UNSUPPORTED;
-    }
+    if ((rc = check_array_options(opt))) return rc;
     Slot &s = h->slots[slot];
     cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
     std::vector<TableArgs> tabs(1);
     TableArgs &a = tabs[0];
-    memset(&a.tv, 0, sizeof a.tv);
-    memset(&a.ov, 0, sizeof a.ov);
-    a.tv.kind = 1;
-    a.tv.n = n;
-    a.tv.t = d_t;
-    a.tv.data = reinterpret_cast<const double2 *>(d_data);
-    a.ov.kind = 1;
-    a.ov.out = reinterpret_cast<double2 *>(d_out);
+    array_views(n, d_t, reinterpret_cast<const double2 *>(d_data), reinterpret_cast<double2 *>(d_out), a);
     a.wrows = nwindow;
     a.d_state_in = d_state;
     a.d_params = d_params;
@@ -1218,137 +1320,8 @@ int gppd_submit_table_f32(gppd_handle h, int slot, int64_t n, const int32_t *tim
         g_last_error = "process_table_f32: bad slot, null buffer or n < 2";
         return GPPD_ERR_ARG;
     }
-    gppd_options o;
-    memset(&o, 0, sizeof o);
-    if (opt) o = *opt;
-    centre_mode(o, offsets != nullptr);
-    int64_t wrows = n, nwin = 1;
-    if ((rc = gppd_table_windows(n, time_us, mjd, window_s, &wrows, &nwin))) return rc;
-    size_t nfits = (size_t)nwin * NDIODE;
-    Slot &s = h->slots[slot];
-    cudaStream_t st = s.stream;
-    CK(cudaStreamSynchronize(st));  // slot reuse: previous table of this slot must be done
-    size_t vbytes = sizeof(float) * 80 * (size_t)n;
-    size_t obytes = sizeof(float) * ((o.flags & GPPD_KEEPRAW) ? 144 : 80) * (size_t)n;
-    if ((rc = s.time.ensure(sizeof(int32_t) * (size_t)n))) return rc;
-    if ((rc = s.volt.ensure(vbytes))) return rc;
-    if ((rc = s.volt_out.ensure(obytes))) return rc;
-    if ((rc = s.params.ensure(sizeof(double) * 6 * nfits))) return rc;
-    if ((rc = s.chi2.ensure(sizeof(double) * nfits))) return rc;
-    if ((rc = s.info.ensure(sizeof(int) * GPPD_INFO_STRIDE * nfits))) return rc;
-    if ((rc = s.state_out.ensure((size_t)n))) return rc;
-    if ((rc = s.offsets.ensure(sizeof(double) * 80))) return rc;
-    CK(cudaMemcpyAsync(s.time.p, time_us, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(s.volt.p, volt, vbytes, cudaMemcpyHostToDevice, st));
-    if (offsets)
-        CK(cudaMemcpyAsync(s.offsets.p, offsets, sizeof(double) * 80, cudaMemcpyHostToDevice, st));
-    std::vector<TableArgs> tabs(1);
-    TableArgs &a = tabs[0];
-    table_views(n, mjd, s.time.as<int32_t>(), s.volt.as<float>(),
-                offsets ? s.offsets.as<double>() : nullptr, s.volt_out.as<float>(), o.flags, a);
-    a.wrows = wrows;
-    const bool faint = timer1 && timer2 && n1 > 0 && n2 > 0;
-    a.timer1 = timer1;
-    a.timer2 = timer2;
-    a.n1 = faint ? n1 : 0;
-    a.n2 = faint ? n2 : 0;
-    a.d_params = s.params.as<double>();
-    a.d_chi2 = s.chi2.as<double>();
-    a.d_info = s.info.as<int>();
-    a.d_state_out = s.state_out.as<int8_t>();
-    if ((rc = run_tables(h, s, st, tabs, o))) return rc;
-    CK(cudaMemcpyAsync(volt_out, s.volt_out.p, obytes, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(params, s.params.p, sizeof(double) * 6 * nfits, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(chi2, s.chi2.p, sizeof(double) * nfits, cudaMemcpyDeviceToHost, st));
-    if (info)
-        CK(cudaMemcpyAsync(info, s.info.p, sizeof(int) * GPPD_INFO_STRIDE * nfits,
-                           cudaMemcpyDeviceToHost, st));
-    if (state_out && faint)
-        CK(cudaMemcpyAsync(state_out, s.state_out.p, (size_t)n, cudaMemcpyDeviceToHost, st));
-    return GPPD_OK;
-}
-
-// The record path of gppd_submit_fits_rows / gppd_file_submit: upload (unless the records are
-// already in s.rows: `rows_uploaded`), unpack, the batch, pack, download.  `first2` = the first
-// two records on the host (for the --window arithmetic, :192).
-static int submit_rows_core(gppd_handle h, int slot, int64_t n, const void *rows, bool rows_uploaded,
-                            const unsigned char *first2, int64_t row_bytes, int64_t time_off,
-                            int64_t volt_off, double mjd, const double *offsets, const double *timer1,
-                            int64_t n1, const double *timer2, int64_t n2, double window_s,
-                            const gppd_options *opt, void *rows_out, double *params, double *chi2,
-                            int32_t *info, int8_t *state_out, int64_t *nfits_out) {
-    int rc;
-    if (slot < 0 || slot >= NSLOTS || !first2 || !rows_out || !params || !chi2 || n < 2 ||
-        time_off < 0 || volt_off < 0 || time_off + 4 > row_bytes || volt_off + 320 > row_bytes ||
-        (time_off + 4 > volt_off && time_off < volt_off + 320)) {
-        g_last_error = "fits rows: bad slot, null buffer, n < 2 or fields outside the record";
-        return GPPD_ERR_ARG;
-    }
-    gppd_options o;
-    memset(&o, 0, sizeof o);
-    if (opt) o = *opt;
-    centre_mode(o, offsets != nullptr);
-    o.flags &= ~GPPD_BIG_ENDIAN;    // the unpack pass delivers little-endian arrays
-    const int out_floats = (o.flags & GPPD_KEEPRAW) ? 144 : 80;
-    const int64_t row_bytes_out = row_bytes + 4 * (out_floats - 80);
-    // TIME of the first two records (host side), for the --window arithmetic (:192)
-    int32_t t01[2];
-    for (int k = 0; k < 2; ++k) {
-        const unsigned char *p = first2 + k * row_bytes + time_off;
-        t01[k] = (int32_t)(((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | p[3]);
-    }
-    int64_t wrows = n, nwin = 1;
-    if ((rc = gppd_table_windows(2, t01, mjd, window_s, &wrows, &nwin))) return rc;
-    if (!(window_s > 0.0)) wrows = n;
-    nwin = gppd_num_windows(n, wrows);
-    size_t nfits = (size_t)nwin * NDIODE;
-    if (nfits_out) *nfits_out = (int64_t)nfits;
-    Slot &s = h->slots[slot];
-    cudaStream_t st = s.stream;
-    if (!rows_uploaded) CK(cudaStreamSynchronize(st));  // slot reuse: previous table of this slot must be done
-    if ((rc = s.rows.ensure((size_t)n * (size_t)row_bytes))) return rc;
-    if ((rc = s.rows_out.ensure((size_t)n * (size_t)row_bytes_out))) return rc;
-    if ((rc = s.time.ensure(sizeof(int32_t) * (size_t)n))) return rc;
-    if ((rc = s.volt.ensure(sizeof(float) * 80 * (size_t)n))) return rc;
-    if ((rc = s.volt_out.ensure(sizeof(float) * out_floats * (size_t)n))) return rc;
-    if ((rc = s.params.ensure(sizeof(double) * 6 * nfits))) return rc;
-    if ((rc = s.chi2.ensure(sizeof(double) * nfits))) return rc;
-    if ((rc = s.info.ensure(sizeof(int) * GPPD_INFO_STRIDE * nfits))) return rc;
-    if ((rc = s.state_out.ensure((size_t)n))) return rc;
-    if ((rc = s.offsets.ensure(sizeof(double) * 80))) return rc;
-    if (!rows_uploaded)
-        CK(cudaMemcpyAsync(s.rows.p, rows, (size_t)n * (size_t)row_bytes, cudaMemcpyHostToDevice, st));
-    if (offsets)
-        CK(cudaMemcpyAsync(s.offsets.p, offsets, sizeof(double) * 80, cudaMemcpyHostToDevice, st));
-    Launcher L{st, &h->launches};
-    launch_unpack_rows(L, s.rows.p, n, row_bytes, time_off, volt_off, s.time.as<int32_t>(), s.volt.as<float>());
-    std::vector<TableArgs> tabs(1);
-    TableArgs &a = tabs[0];
-    table_views(n, mjd, s.time.as<int32_t>(), s.volt.as<float>(),
-                offsets ? s.offsets.as<double>() : nullptr, s.volt_out.as<float>(), o.flags, a);
-    a.wrows = wrows;
-    const bool faint = timer1 && timer2 && n1 > 0 && n2 > 0;
-    a.timer1 = timer1;
-    a.timer2 = timer2;
-    a.n1 = faint ? n1 : 0;
-    a.n2 = faint ? n2 : 0;
-    a.d_params = s.params.as<double>();
-    a.d_chi2 = s.chi2.as<double>();
-    a.d_info = s.info.as<int>();
-    a.d_state_out = s.state_out.as<int8_t>();
-    if ((rc = run_tables(h, s, st, tabs, o))) return rc;
-    launch_pack_rows(L, s.rows.p, n, row_bytes, volt_off, s.volt_out.as<float>(), out_floats, s.rows_out.p,
-                     row_bytes_out);
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(rows_out, s.rows_out.p, (size_t)n * (size_t)row_bytes_out, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(params, s.params.p, sizeof(double) * 6 * nfits, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(chi2, s.chi2.p, sizeof(double) * nfits, cudaMemcpyDeviceToHost, st));
-    if (info)
-        CK(cudaMemcpyAsync(info, s.info.p, sizeof(int) * GPPD_INFO_STRIDE * nfits,
-                           cudaMemcpyDeviceToHost, st));
-    if (state_out && faint)
-        CK(cudaMemcpyAsync(state_out, s.state_out.p, (size_t)n, cudaMemcpyDeviceToHost, st));
-    return GPPD_OK;
+    return stage_table(h, slot, n, time_us, volt, nullptr, false, 0, 0, 0, mjd, offsets, timer1, n1, timer2, n2,
+                       window_s, opt, volt_out, params, chi2, info, state_out);
 }
 
 int gppd_submit_fits_rows(gppd_handle h, int slot, int64_t n, const void *rows, int64_t row_bytes,
@@ -1358,14 +1331,12 @@ int gppd_submit_fits_rows(gppd_handle h, int slot, int64_t n, const void *rows, 
                           double *chi2, int32_t *info, int8_t *state_out) {
     int rc = check_handle(h);
     if (rc) return rc;
-    if (!rows) {
-        g_last_error = "submit_fits_rows: null buffer";
+    if (slot < 0 || slot >= NSLOTS || !rows || !rows_out || !params || !chi2 || n < 2) {
+        g_last_error = "submit_fits_rows: bad slot, null buffer or n < 2";
         return GPPD_ERR_ARG;
     }
-    std::lock_guard<std::mutex> lk(h->launch_mutex);
-    return submit_rows_core(h, slot, n, rows, false, reinterpret_cast<const unsigned char *>(rows), row_bytes,
-                            time_off, volt_off, mjd, offsets, timer1, n1, timer2, n2, window_s, opt, rows_out,
-                            params, chi2, info, state_out, nullptr);
+    return stage_table(h, slot, n, nullptr, nullptr, rows, false, row_bytes, time_off, volt_off, mjd, offsets,
+                       timer1, n1, timer2, n2, window_s, opt, rows_out, params, chi2, info, state_out);
 }
 
 // ---------------------------------------------------------------------------
@@ -1426,26 +1397,19 @@ int file_reader(gppd_handle h, int slot) {
     }
     close(fd);
     // number of fits (windows x 32) -> the small pinned result buffers
-    int32_t t01[2];
-    for (int k = 0; k < 2; ++k) {
-        const unsigned char *p = f.rows.as<unsigned char>() + k * f.row_bytes + f.time_off;
-        t01[k] = (int32_t)(((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | p[3]);
-    }
     int64_t wrows = f.n, nwin = 1;
-    if ((rc = gppd_table_windows(2, t01, f.mjd, f.window_s, &wrows, &nwin))) return rc;
-    if (!(f.window_s > 0.0)) wrows = f.n;
-    nwin = gppd_num_windows(f.n, wrows);
+    if ((rc = record_windows(f.n, f.rows.as<unsigned char>(), f.row_bytes, f.time_off, f.volt_off, f.mjd,
+                             f.window_s, wrows, nwin)))
+        return rc;
     f.nfits = nwin * NDIODE;
     if ((rc = f.params.ensure(sizeof(double) * 6 * (size_t)f.nfits))) return rc;
     if ((rc = f.chi2.ensure(sizeof(double) * (size_t)f.nfits))) return rc;
     if ((rc = f.info.ensure(sizeof(int32_t) * GPPD_INFO_STRIDE * (size_t)f.nfits))) return rc;
-    std::lock_guard<std::mutex> lk(h->launch_mutex);
-    return submit_rows_core(h, slot, f.n, nullptr, true, f.rows.as<unsigned char>(), f.row_bytes, f.time_off,
-                            f.volt_off, f.mjd, f.have_offsets ? f.offsets : nullptr,
-                            f.faint ? f.timer1.data() : nullptr, (int64_t)f.timer1.size(),
-                            f.faint ? f.timer2.data() : nullptr, (int64_t)f.timer2.size(), f.window_s, &f.opt,
-                            f.rows_out.p, f.params.as<double>(), f.chi2.as<double>(), f.info.as<int32_t>(),
-                            f.state.as<int8_t>(), nullptr);
+    return stage_table(h, slot, f.n, nullptr, nullptr, f.rows.p, true, f.row_bytes, f.time_off, f.volt_off, f.mjd,
+                       f.have_offsets ? f.offsets : nullptr, f.faint ? f.timer1.data() : nullptr,
+                       (int64_t)f.timer1.size(), f.faint ? f.timer2.data() : nullptr, (int64_t)f.timer2.size(),
+                       f.window_s, &f.opt, f.rows_out.p, f.params.as<double>(), f.chi2.as<double>(),
+                       f.info.as<int32_t>(), f.state.as<int8_t>());
 }
 
 int write_all(int fd, const void *buf, size_t len, const std::string &path) {
@@ -1730,20 +1694,17 @@ int gppd_process_tables_f32_dev(gppd_handle h, int slot, void *stream, int64_t n
         g_last_error = "process_tables_f32_dev: bad slot or null array";
         return GPPD_ERR_ARG;
     }
-    gppd_options o;
-    memset(&o, 0, sizeof o);
-    if (opt) o = *opt;
-    centre_mode(o, d_offsets != nullptr);
-    Slot &s = h->slots[slot];
-    cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
-    std::vector<TableArgs> tabs((size_t)ntables);
     for (int64_t t = 0; t < ntables; ++t) {
-        TableArgs &a = tabs[(size_t)t];
-        if (!d_time_us[t] || !d_volt[t] || !d_volt_out[t] || !d_params[t] || !d_chi2[t] ||
-            n[t] < 2) {
+        if (!d_time_us[t] || !d_volt[t] || !d_volt_out[t] || !d_params[t] || !d_chi2[t] || n[t] < 2) {
             g_last_error = "process_tables_f32_dev: null table buffer or n < 2";
             return GPPD_ERR_ARG;
         }
+    }
+    gppd_options o;
+    if ((rc = table_options(opt, d_offsets != nullptr, o))) return rc;
+    std::vector<TableArgs> tabs((size_t)ntables);
+    for (int64_t t = 0; t < ntables; ++t) {
+        TableArgs &a = tabs[(size_t)t];
         table_views(n[t], mjd[t], d_time_us[t], d_volt[t], d_offsets, d_volt_out[t], o.flags, a);
         a.wrows = nwindow_rows ? nwindow_rows[t] : 0;
         const bool faint = timer1 && timer2 && n1 && n2 && timer1[t] && timer2[t] && n1[t] > 0 &&
@@ -1757,34 +1718,7 @@ int gppd_process_tables_f32_dev(gppd_handle h, int slot, void *stream, int64_t n
         a.d_info = d_info ? d_info[t] : nullptr;
         a.d_state_out = d_state_out ? d_state_out[t] : nullptr;
     }
-    // FAINT tables and bright tables as two concurrent chains (results do not depend
-    // on the batching: all partial sums are over fixed row segments)
-    if (o.flags & GPPD_CENTER_ELLIPSE) return run_batch_ellipse(h, s, st, tabs, o);
-    std::vector<TableArgs> faint, bright;
-    for (TableArgs &a : tabs) (a.n1 > 0 ? faint : bright).push_back(a);
-    // (the fit's latency-bound tail and the HBM-bound demodulation of one chain overlap the
-    // issue-bound harmonic pass of the other: measured +8 % on the 100-table night.  Each
-    // pass is then two launches per batch; gppd_pass_times adds their durations.
-    // GPPD_SPLIT_CHAINS=0 or gppd_set_split_chains(h, 0) keeps one launch sequence.)
-    // (not for batches of very many small fits: there the one-thread-per-fit solver dominates
-    // and two concurrent launches of it are slower than one -- measured, 20 tables: 5 000-row
-    // windows (12 800 fits) 3.3 against 4.3 ms, 2 000-row windows (32 000 fits) 5.0 against 4.3)
-    long long nfits_total = 0;
-    for (const TableArgs &a : tabs) {
-        const long long w = (a.wrows <= 0 || a.wrows >= a.tv.n) ? a.tv.n : a.wrows;
-        nfits_total += (a.tv.n + w - 1) / w * NDIODE;
-    }
-    if (faint.empty() || bright.empty() || !h->split_chains || nfits_total > 16384 ||
-        (o.flags & GPPD_CENTER_EMPIRICAL))
-        return run_batch(h, s, st, tabs, &o, nullptr, false);
-    Slot &sb = h->aux[slot];
-    CK(cudaEventRecord(sb.fork, st));
-    CK(cudaStreamWaitEvent(sb.stream, sb.fork, 0));
-    if ((rc = run_batch(h, sb, sb.stream, faint, &o, nullptr, false))) return rc;
-    if ((rc = run_batch(h, s, st, bright, &o, nullptr, false))) return rc;
-    CK(cudaEventRecord(sb.join, sb.stream));
-    CK(cudaStreamWaitEvent(st, sb.join, 0));
-    return GPPD_OK;
+    return run_tables(h, slot, stream ? (cudaStream_t)stream : h->slots[slot].stream, tabs, o);
 }
 
 int gppd_process_table_f32_dev(gppd_handle h, int slot, void *stream, int64_t n,
