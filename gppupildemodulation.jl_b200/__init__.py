@@ -13,6 +13,6 @@ from . import sharding, synthetic  # noqa: F401
 from ._lib import GppdError, Handle, build, default_handle  # noqa: F401
 from .api import (D1, D2, D3, D4, FC, FT, HIGH, LOW, M_2PI, NORMAL, OFF, SC,  # noqa: F401
                   TRANSIENT, Diode, FaintStates, MetState, ModulationNoOffsets,
-                  ModulationWithOffsets, Side, buildfaintparameters, buildstates,
+                  ModulationWithOffsets, Side, buildfaintparameters, buildstates, covariances,
                   demodulateall, ellipse_keys, ellipses, idx, process_table, processmetrology, read_stefan_file,
-                  table_windows)
+                  table_windows, uncertainty_keys, window_uncertainty_columns)

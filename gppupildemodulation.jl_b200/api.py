@@ -133,13 +133,14 @@ def buildstates(faintstates: FaintStates, timestamp, lag: int = 0, preswitchdela
 
 
 def _options(onlyhigh=False, fitoffsets=False, recenter=True, keepraw=False, init="auto",
-             method="auto", maxfun=0, empirical=False, groups=0, fp32=False, ellipse=False) -> Options:
+             method="auto", maxfun=0, empirical=False, groups=0, fp32=False, ellipse=False,
+             covariance=False) -> Options:
     o = Options()
     o.group_mask = int(groups) & 0xff
     o.flags = ((_lib.ONLYHIGH if onlyhigh else 0) | (_lib.FITOFFSETS if fitoffsets else 0) |
                (0 if recenter else _lib.NO_RECENTER) | (_lib.KEEPRAW if keepraw else 0) |
                (_lib.CENTER_EMPIRICAL if empirical else 0) | (_lib.FP32 if fp32 else 0) |
-               (_lib.CENTER_ELLIPSE if ellipse else 0))
+               (_lib.CENTER_ELLIPSE if ellipse else 0) | (_lib.COVARIANCE if covariance else 0))
     o.method = {"auto": _lib.METHOD_AUTO, "direct": _lib.METHOD_DIRECT,
                 "harmonic": _lib.METHOD_HARMONIC}[method]
     o.maxfun = int(maxfun)
@@ -170,7 +171,7 @@ def _params_to_structs(params, fitoffsets):
 def demodulateall(timestamp, data, init="auto", recenter=True, faintparam=None,
                   onlyhigh=False, fitoffsets=False, preswitchdelay=0.01, postwitchdelay=0.3,
                   *, raw=False, nwindow=0, method="auto", maxfun=0, return_info=False,
-                  return_trace=False, handle=None, groups=0):
+                  return_trace=False, handle=None, groups=0, return_cov=False, rhoend=0.0):
     """demodulateall(timestamp, data; init, recenter, faintparam, onlyhigh,
     fitoffsets, preswitchdelay, postwitchdelay) -> (output, param, likelihood)
     (src/Modulation.jl:344-435).
@@ -182,7 +183,9 @@ def demodulateall(timestamp, data, init="auto", recenter=True, faintparam=None,
     ``gppd_options.group_mask`` (bit g = (telescope, side) group g of
     src/Modulation.jl:387; 0 = all): only those groups' columns, params and chi2 entries
     are computed, the rest of the returned arrays is unspecified -- see
-    ``sharding.gather_groups``.
+    ``sharding.gather_groups``.  ``return_cov`` (GPPD_COVARIANCE) appends the
+    (nwin*32, 6, 6) parameter covariances (``covariances``); ``rhoend`` is NEWUOA's final
+    trust-region radius (0: the reference's 1e-3).
     """
     h = handle or _lib.default_handle()
     t = np.ascontiguousarray(timestamp, dtype=np.float64)
@@ -199,7 +202,8 @@ def demodulateall(timestamp, data, init="auto", recenter=True, faintparam=None,
         if state.shape != (n,):
             raise ValueError("state and time must have the same number of lines")
     o = _options(onlyhigh=onlyhigh, fitoffsets=fitoffsets, recenter=recenter, init=init,
-                 method=method, maxfun=maxfun, groups=groups)
+                 method=method, maxfun=maxfun, groups=groups, covariance=return_cov)
+    o.rhoend = float(rhoend)
     nwin = int(lib().gppd_num_windows(n, int(nwindow)))
     out = np.empty((n, 40), dtype=np.complex128, order="F")
     params = np.empty((nwin * 32, 6))
@@ -215,7 +219,18 @@ def demodulateall(timestamp, data, init="auto", recenter=True, faintparam=None,
         res.append(info)
     if return_trace:
         res.append(trace)
+    if return_cov:
+        res.append(covariances(h, 0, nwin * 32))
     return tuple(res)
+
+
+def covariances(handle=None, slot=0, nfits=32):
+    """The (nfits, 6, 6) parameter covariances of the last GPPD_COVARIANCE call on pipeline
+    slot ``slot`` (``gppd_covariances``), in params order (c.re, c.im, a.re, a.im, b, phi)."""
+    h = handle or _lib.default_handle()
+    cov = np.empty((int(nfits), 6, 6))
+    check(lib().gppd_covariances(h.raw, int(slot), int(nfits), ptr(cov)))
+    return cov
 
 
 def table_windows(time_us, mjd, window):
@@ -231,7 +246,7 @@ def table_windows(time_us, mjd, window):
 def process_table(time_us, volt, mjd, offsets=None, faintparam: FaintStates | None = None,
                   window=None, keepraw=False, onlyhigh=False, method="auto", maxfun=0,
                   handle=None, centres_out=None, fp32=False, ellipses_out=None,
-                  ellipse_status_out=None):
+                  ellipse_status_out=None, cov_out=None):
     """Array-level fast path (C ABI ``gppd_process_table_f32``): returns
     (volt_out float32 (N, 80|144), params (nwin*32, 6), chi2, info, state|None).
     ``offsets``: (40,) complex128 centres, ``None`` (fit the centres) or ``True``
@@ -242,7 +257,8 @@ def process_table(time_us, volt, mjd, offsets=None, faintparam: FaintStates | No
     fitted on the device, maps every channel onto a circle before the fit (include/gppd.h);
     ``ellipses_out`` ((40, 6) float64: x0, y0, r, alpha, m21, m22) and
     ``ellipse_status_out`` ((40,) int32: 2 ellipse, 1 circle only, 0 neither) then receive
-    the maps."""
+    the maps.  ``cov_out``, a (nwin*32, 6, 6) float64 array, turns on GPPD_COVARIANCE and
+    receives the parameter covariances."""
     h = handle or _lib.default_handle()
     tu = np.ascontiguousarray(time_us, dtype=np.int32)
     v = np.ascontiguousarray(volt, dtype=np.float32)
@@ -257,7 +273,7 @@ def process_table(time_us, volt, mjd, offsets=None, faintparam: FaintStates | No
            else np.ascontiguousarray(offsets, dtype=np.complex128))
     _, nwin = table_windows(tu, mjd, window)
     o = _options(onlyhigh=onlyhigh, keepraw=keepraw, method=method, maxfun=maxfun,
-                 empirical=empirical, fp32=fp32, ellipse=ellipse)
+                 empirical=empirical, fp32=fp32, ellipse=ellipse, covariance=cov_out is not None)
     vout = np.empty((n, 144 if keepraw else 80), dtype=np.float32)
     params = np.empty((nwin * 32, 6))
     chi2 = np.empty(nwin * 32)
@@ -281,6 +297,8 @@ def process_table(time_us, volt, mjd, offsets=None, faintparam: FaintStates | No
             ellipses_out[:] = e[0]
         if ellipse_status_out is not None:
             ellipse_status_out[:] = st[0]
+    if cov_out is not None:
+        cov_out[...] = covariances(h, 0, nwin * 32).reshape(cov_out.shape)
     return vout, params, chi2, info, state
 
 
@@ -338,6 +356,55 @@ def demodulation_keys(params, fitoffsets: bool) -> dict:
     return hdr
 
 
+def uncertainties(params, cov) -> dict:
+    """One-sigma uncertainties of the reported quantities from the (nfits, 6) parameters and
+    their (nfits, 6, 6) covariances: |a| and arg a by the delta method on the a block
+    (d|a| = (a.re, a.im) / |a|, d arg a = (-a.im, a.re) / |a|^2), b, phi, x0 = c.re and
+    y0 = c.im from the diagonal.  (nfits,) arrays keyed ABSA, ARGA, B, PHI, X0, Y0."""
+    P = np.asarray(params, dtype=np.float64).reshape(-1, 6)
+    V = np.asarray(cov, dtype=np.float64).reshape(-1, 6, 6)
+    ar, ai = P[:, 2], P[:, 3]
+    r2 = ar * ar + ai * ai
+    vrr, vri, vii = V[:, 2, 2], V[:, 2, 3], V[:, 3, 3]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        var_abs = (ar * ar * vrr + 2 * ar * ai * vri + ai * ai * vii) / r2
+        var_arg = (ai * ai * vrr - 2 * ar * ai * vri + ar * ar * vii) / (r2 * r2)
+        diag = np.sqrt(np.diagonal(V, axis1=1, axis2=2))
+    return {"ABSA": np.sqrt(var_abs), "ARGA": np.sqrt(var_arg), "B": diag[:, 4], "PHI": diag[:, 5],
+            "X0": diag[:, 0], "Y0": diag[:, 1]}
+
+
+def uncertainty_keys(params, cov, fitoffsets: bool) -> dict:
+    """The whole-file header keywords of ``--uncertainty``, next to those of
+    ``demodulation_keys``: DEMODULATION {AMPLITUDE ABS|AMPLITUDE ARG|SIN AMPLITUDE|SIN PHASE}
+    ERR {FT|SC} T{1-4} D{1-4}, and CENTER {X0|Y0} ERR where the CENTER keys are written."""
+    u = uncertainties(params, cov)
+    hdr = {}
+    for s in (Side.FT, Side.SC):
+        for j in range(1, 5):
+            for d in (Diode.D1, Diode.D2, Diode.D3, Diode.D4):
+                ch = s + (d - 1) + (j - 1) * 4      # idx() - 1, src/Modulation.jl:17-22
+                suffix = f"{s.name} T{j} {d.name}"
+                if fitoffsets:
+                    hdr[f"DEMODULATION CENTER X0 ERR {suffix}"] = float(u["X0"][ch])
+                    hdr[f"DEMODULATION CENTER Y0 ERR {suffix}"] = float(u["Y0"][ch])
+                hdr[f"DEMODULATION AMPLITUDE ABS ERR {suffix}"] = float(u["ABSA"][ch])
+                hdr[f"DEMODULATION AMPLITUDE ARG ERR {suffix}"] = float(u["ARGA"][ch])
+                hdr[f"DEMODULATION SIN AMPLITUDE ERR {suffix}"] = float(u["B"][ch])
+                hdr[f"DEMODULATION SIN PHASE ERR {suffix}"] = float(u["PHI"][ch])
+    return hdr
+
+
+def window_uncertainty_columns(params, cov, n: int, wrows: int, nwin: int, fitoffsets: bool) -> dict:
+    """The per-row columns of ``--uncertainty`` in window mode, next to those of
+    ``window_columns``: ABSA_ERR, ARGA_ERR, B_ERR, PHI_ERR (and X0_ERR, Y0_ERR), each
+    window's values broadcast over its rows, Float32 (n, 32)."""
+    u = uncertainties(params, cov)
+    rows = np.minimum(np.arange(n) // wrows, nwin - 1)
+    names = (("X0", "Y0") if fitoffsets else ()) + ("ABSA", "ARGA", "B", "PHI")
+    return {k + "_ERR": u[k].reshape(nwin, 32)[rows].astype(np.float32) for k in names}
+
+
 def window_columns(params, n: int, wrows: int, nwin: int, fitoffsets: bool) -> dict:
     """The per-row parameter tables of window mode (src/GPPupilDemodulation.jl:209-247):
     each window's values broadcast over its rows, Float32 (n, 32)."""
@@ -362,7 +429,7 @@ def window_columns(params, n: int, wrows: int, nwin: int, fitoffsets: bool) -> d
 
 def processmetrology(table, mjd, window=None, faintparam: FaintStates | None = None,
                      keepraw=False, verb=False, onlyhigh=False, offsets=True, handle=None,
-                     method="auto"):
+                     method="auto", uncertainty=False):
     """processmetrology(metrologyhdu, mjd; window, faintparam, keepraw, verb,
     onlyhigh, offsets) -> (table, hdr)   (src/GPPupilDemodulation.jl:128-255).
 
@@ -373,7 +440,9 @@ def processmetrology(table, mjd, window=None, faintparam: FaintStates | None = N
     channel over the HIGH samples of a FAINT table, all samples otherwise.  The
     reference throws here because its ``Circle`` is undefined; this is the algebraic
     circle fit that call stands for) or ``"ellipse"`` (one ellipse per channel, see
-    ``process_table``; the header then records the maps, ``ellipse_keys``)."""
+    ``process_table``; the header then records the maps, ``ellipse_keys``).
+    ``uncertainty`` adds the one-sigma uncertainties (``uncertainty_keys``,
+    ``window_uncertainty_columns``)."""
     out = dict(table)
     hdr = {}
     ell = np.empty((40, 6)) if isinstance(offsets, str) and offsets == "ellipse" else None
@@ -384,15 +453,21 @@ def processmetrology(table, mjd, window=None, faintparam: FaintStates | None = N
     else:
         off = None if offsets is False else np.asarray(offsets, dtype=np.complex128)
     fitoffsets = off is None
+    wrows, nwin = table_windows(table["TIME"], mjd, window)
+    cov = np.empty((nwin * 32, 6, 6)) if uncertainty else None
     vout, params, chi2, info, state = process_table(
         table["TIME"], table["VOLT"], mjd, offsets=off, faintparam=faintparam, window=window,
-        keepraw=keepraw, onlyhigh=onlyhigh, handle=handle, method=method, ellipses_out=ell)
+        keepraw=keepraw, onlyhigh=onlyhigh, handle=handle, method=method, ellipses_out=ell,
+        cov_out=cov)
     n = vout.shape[0]
     if window is None:
         hdr.update(demodulation_keys(params, fitoffsets))
+        if uncertainty:
+            hdr.update(uncertainty_keys(params, cov, fitoffsets))
     else:
-        wrows, nwin = table_windows(table["TIME"], mjd, window)
         out.update(window_columns(params, n, wrows, nwin, fitoffsets))
+        if uncertainty:
+            out.update(window_uncertainty_columns(params, cov, n, wrows, nwin, fitoffsets))
         if state is not None:
             out["STATE"] = state.astype(np.int8)   # :248
     if ell is not None:

@@ -36,8 +36,8 @@ import numpy as np
 
 from . import _lib, fits
 from .sharding import partition_files
-from .api import (_options, buildfaintparameters, demodulation_keys, ellipse_keys, ellipses,
-                  read_stefan_file, window_columns)
+from .api import (_options, buildfaintparameters, covariances, demodulation_keys, ellipse_keys, ellipses,
+                  read_stefan_file, uncertainty_keys, window_columns, window_uncertainty_columns)
 
 SUFFIXES = (".fits", ".fits.gz", "fits.Z")      # src/GPPupilDemodulation.jl:14
 log = logging.getLogger("GPPupilDemodulation")
@@ -61,6 +61,9 @@ def build_parser() -> argparse.ArgumentParser:
                         "(offset and ellipse correction of each channel, fitted per file)")
     p.add_argument("--window", "-w", type=float, default=0.0,
                    help="Compute demodulation on non overlapping window of WINDOW second")
+    p.add_argument("--uncertainty", action="store_true",
+                   help="also write the one-sigma uncertainty of every fitted quantity (ERR header keys, "
+                        "*_ERR columns in window mode)")
     p.add_argument("--dir", "-d", default=os.getcwd(), help="output folder")
     p.add_argument("--rank", type=int, default=int(os.environ.get("RANK", "0")), help=argparse.SUPPRESS)
     p.add_argument("--world", type=int, default=int(os.environ.get("WORLD_SIZE", "1")), help=argparse.SUPPRESS)
@@ -124,7 +127,7 @@ def _plan_file(filename, args, folder):
 class NightScheduler:
     """Files -> pipeline slots of one handle (one GPU)."""
 
-    def __init__(self, handle, offsets, onlyhigh, method="auto"):
+    def __init__(self, handle, offsets, onlyhigh, method="auto", uncertainty=False):
         self.h, self.L = handle, _lib.lib()
         self.empirical = offsets is True       # --center empirical: centres fitted on the device
         # --center ellipse: one ellipse per channel fitted and applied on the device
@@ -132,6 +135,7 @@ class NightScheduler:
         self.offsets = (None if (offsets is None or self.empirical or self.ellipse)
                         else np.ascontiguousarray(offsets, dtype=np.complex128))
         self.onlyhigh, self.method = onlyhigh, method
+        self.uncertainty = uncertainty         # --uncertainty: parameter covariances (GPPD_COVARIANCE)
         self.nslots = handle.num_slots
         self.busy = [None] * self.nslots       # (job, buffers) per slot
         self.pinned = [dict() for _ in range(self.nslots)]
@@ -175,7 +179,7 @@ class NightScheduler:
             wrows = w.value
             nwin = (n + wrows - 1) // wrows
         o = _options(onlyhigh=self.onlyhigh, keepraw=job.keepraw, method=self.method,
-                     empirical=self.empirical, ellipse=self.ellipse)
+                     empirical=self.empirical, ellipse=self.ellipse, covariance=self.uncertainty)
         fp = job.faintparam
         t1 = fp.timer1 if fp is not None else None
         t2 = fp.timer2 if fp is not None else None
@@ -217,6 +221,7 @@ class NightScheduler:
             return self._finish_native(slot, job, b)
         _lib.check(self.L.gppd_wait(self.h.raw, slot))
         b["ell"] = self._ellipses(slot)
+        b["cov"] = self._covariances(slot, b["nwin"])
         # the slot's staging buffers are reused by the next file: take the results out
         b = dict(b, rows_out=b["rows_out"].copy(), params=b["params"].copy(), chi2=b["chi2"].copy(),
                  state=None if b["state"] is None else b["state"].copy())
@@ -225,6 +230,10 @@ class NightScheduler:
     def _ellipses(self, slot):
         """The (40, 6) maps of the slot's last file (--center ellipse), else None."""
         return ellipses(self.h, slot, 1)[0][0] if self.ellipse else None
+
+    def _covariances(self, slot, nwin):
+        """The (nwin*32, 6, 6) covariances of the slot's last file (--uncertainty), else None."""
+        return covariances(self.h, slot, nwin * 32) if self.uncertainty else None
 
     def _table_edits(self, job, b, n):
         """(header keys, new columns, extra per-row bytes or None) of the output table
@@ -235,10 +244,15 @@ class NightScheduler:
             keys += list(ellipse_keys(b["ell"]).items())
         if job.window is None:
             keys += list(demodulation_keys(b["params"], fitoffsets).items())
+            if b["cov"] is not None:
+                keys += list(uncertainty_keys(b["params"], b["cov"], fitoffsets).items())
         else:
             cols = window_columns(b["params"], n, b["wrows"], b["nwin"], fitoffsets)
+            if b["cov"] is not None:
+                cols.update(window_uncertainty_columns(b["params"], b["cov"], n, b["wrows"], b["nwin"], fitoffsets))
             parts = []
-            for name in ("ABSA", "ARGA", "B", "PHI", "X0", "Y0"):
+            for name in ("ABSA", "ARGA", "B", "PHI", "X0", "Y0",
+                         "ABSA_ERR", "ARGA_ERR", "B_ERR", "PHI_ERR", "X0_ERR", "Y0_ERR"):
                 if name in cols:
                     parts.append(cols[name].astype(">f4").view(np.uint8).reshape(n, 128))
                     newcols.append((name, "32E", None))
@@ -259,6 +273,7 @@ class NightScheduler:
         _lib.check(self.L.gppd_file_wait(self.h.raw, slot, _lib.ptr(b["params"]), _lib.ptr(b["chi2"]), None,
                                          _lib.ptr(b["state"], _lib._i8p)))
         b["ell"] = self._ellipses(slot)
+        b["cov"] = self._covariances(slot, nwin)
         keys, newcols, extra = self._table_edits(job, b, n)
         met = job.hdus[job.imet]
         rb_new = b["rb_out"] + (0 if extra is None else extra.shape[1])
@@ -367,7 +382,7 @@ def main(argv=None) -> int:
         raise SystemExit(f"unknown --center {args.center}")
     mine = partition_files(files, args.rank, args.world)   # no communication between ranks
     handle = _lib.Handle(args.device)
-    sched = NightScheduler(handle, offsets, args.onlyhigh)
+    sched = NightScheduler(handle, offsets, args.onlyhigh, uncertainty=args.uncertainty)
 
     def jobs():
         # read and gate a few files ahead of the GPU (file reads release the interpreter lock)

@@ -170,6 +170,8 @@ struct Slot {
     // out, FAINT states when the caller keeps none)
     DevBuf etabs, ell, estatus, epart, et, edata, eout, estate;
     int nellipses = 0;              // tables whose ellipses the last batch of this slot fitted
+    DevBuf cov, covpart;            // GPPD_COVARIANCE: [nfits][36] + per-segment partial sums
+    long long ncov = 0;             // fits whose covariances the last batch of this slot computed
     DevBuf params, chi2, info, trace, state_out;
     // batch scratch
     DevBuf state, basis, z, y, thkeys, nvalid, jobs, results;
@@ -337,6 +339,10 @@ int run_batch(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs
     FitOptions fo;
     int method;
     fill_options(opt, fo, method);
+    // the covariance pass is an addition at the end of the sequence: the other passes see the
+    // flag word they see without it
+    const bool want_cov = (fo.flags & GPPD_COVARIANCE) != 0 && !segment_only;
+    fo.flags &= ~GPPD_COVARIANCE;
     const int T = (int)tabs.size();
     if (T <= 0) return GPPD_OK;
     Launcher L{stream, &h->launches};
@@ -485,8 +491,21 @@ int run_batch(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs
         }
     }
 
+    const int CP = want_cov ? cov_max_segments(max_wrows) : 0;
+    if (want_cov) {
+        if (CP > 65535) {
+            g_last_error = "job too long for one launch (more than 65 535 covariance segments)";
+            return GPPD_ERR_ARG;
+        }
+        if ((rc = s.cov.ensure(sizeof(double) * GPPD_COV_STRIDE * (size_t)nfits))) return rc;
+        if ((rc = s.covpart.ensure(sizeof(double) * COV_VALS * NDIODE * (size_t)njobs * CP))) return rc;
+    }
+
     s.ncentres = 0;
-    if (!segment_only) s.nellipses = 0;
+    if (!segment_only) {
+        s.nellipses = 0;
+        s.ncov = 0;
+    }
     if (empirical) {
         // offsets === true: every table gets its own 40 centres, fitted on the device
         if ((rc = s.centres.ensure(sizeof(double2) * NCHAN * (size_t)T))) return rc;
@@ -618,6 +637,14 @@ int run_batch(gppd_handle h, Slot &s, cudaStream_t stream, std::vector<TableArgs
         launch_demod(L, d_tabs, T, max_rows, s.results.as<FitResult>(), fo.flags, arrays);
     }
     DBG(stream, "demod");
+    if (want_cov) {
+        PassScope ps(h, s, stream, GPPD_PASS_EXPORT);
+        launch_covariance(L, d_tabs, s.jobs.as<JobInfo>(), njobs, s.results.as<FitResult>(),
+                          any_state ? s.spart2.as<double>() : nullptr, fo.flags, CP, s.covpart.as<double>(),
+                          s.cov.as<double>());
+        s.ncov = nfits;
+    }
+    DBG(stream, "covariance");
     {
         PassScope ps(h, s, stream, GPPD_PASS_EXPORT);
         launch_export(L, s.exps.as<ExportDesc>(), T, max_jobs * NDIODE, s.results.as<FitResult>(), fo.flags);
@@ -821,8 +848,9 @@ int run_tables(gppd_handle h, int slot, cudaStream_t stream, std::vector<TableAr
         const long long w = (a.wrows <= 0 || a.wrows >= a.tv.n) ? a.tv.n : a.wrows;
         nfits_total += (a.tv.n + w - 1) / w * NDIODE;
     }
+    // (with GPPD_COVARIANCE too: every fit's covariance then lands on the slot gppd_covariances reads)
     if (faint.empty() || bright.empty() || !h->split_chains || nfits_total > 16384 ||
-        (o.flags & GPPD_CENTER_EMPIRICAL))
+        (o.flags & (GPPD_CENTER_EMPIRICAL | GPPD_COVARIANCE)))
         return run_batch(h, s, stream, tabs, &o, nullptr, false);
     Slot &sb = h->aux[slot];
     int rc;
@@ -1074,6 +1102,20 @@ int gppd_ellipses(gppd_handle h, int slot, int64_t ntables, double *ell, int32_t
                   cudaMemcpyDeviceToHost));
     if (status)
         CK(cudaMemcpy(status, s.estatus.p, sizeof(int32_t) * NCHAN * (size_t)ntables, cudaMemcpyDeviceToHost));
+    return GPPD_OK;
+}
+
+int gppd_covariances(gppd_handle h, int slot, int64_t nfits, double *cov) {
+    int rc = check_handle(h);
+    if (rc) return rc;
+    if (slot < 0 || slot >= NSLOTS || !cov || nfits < 1) return GPPD_ERR_ARG;
+    Slot &s = h->slots[slot];
+    if (nfits > s.ncov) {
+        g_last_error = "covariances: the last call on this slot ran without GPPD_COVARIANCE or had fewer fits";
+        return GPPD_ERR_ARG;
+    }
+    CK(cudaStreamSynchronize(s.stream));
+    CK(cudaMemcpy(cov, s.cov.p, sizeof(double) * GPPD_COV_STRIDE * (size_t)nfits, cudaMemcpyDeviceToHost));
     return GPPD_OK;
 }
 

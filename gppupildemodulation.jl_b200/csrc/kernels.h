@@ -96,6 +96,18 @@ void launch_demod(const Launcher &L, const TableDesc *d_tabs, int ntables, long 
 void launch_export(const Launcher &L, const ExportDesc *d_exps, int ntables, int max_fits,
                    const FitResult *d_results, unsigned flags);
 
+// GPPD_COVARIANCE (cov_kernels.cu): per (job, FIXED segment of COV_SEG_ROWS rows) the 21 entries
+// of the upper triangle of H and sum w |r|^2 of each of the job's 32 fits -> d_part
+// [njobs][P][COV_VALS][32]; then per fit the covariance, 36 doubles -> d_cov [nfits][36].
+// d_stats: the per-state (mean, weight) table of the statistics pass (tables with states).
+constexpr int COV_SEG_ROWS = 4096;
+constexpr int COV_SSE = 21;
+constexpr int COV_VALS = 22;
+int cov_max_segments(long long max_rows_per_job);
+void launch_covariance(const Launcher &L, const TableDesc *d_tabs, const JobInfo *d_jobs, int njobs,
+                       const FitResult *d_results, const double *d_stats, unsigned flags, int P, double *d_part,
+                       double *d_cov);
+
 // raw FITS binary-table records <-> dense little-endian TIME / VOLT arrays
 void launch_unpack_rows(const Launcher &L, const void *d_rows, long long n, long long row_bytes,
                         long long time_off, long long volt_off, int32_t *d_time, float *d_volt);

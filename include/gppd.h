@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define GPPD_VERSION 122 /* 0.1.22: + GPPD_FP32, GPPD_CENTER_ELLIPSE / gppd_ellipses; 0.1.21: + gppd_file_* (native ingest); 0.1.20: gppd_options.group_mask, gppd_demodulate_f64_dev (0.1.10: gppd_submit_fits_rows,
+#define GPPD_VERSION 122 /* 0.1.22: + GPPD_COVARIANCE / gppd_covariances, GPPD_FP32, GPPD_CENTER_ELLIPSE / gppd_ellipses; 0.1.21: + gppd_file_* (native ingest); 0.1.20: gppd_options.group_mask, gppd_demodulate_f64_dev (0.1.10: gppd_submit_fits_rows,
                             gppd_centres, gppd_set_split_chains, gppd_debug_harmonics, GPPD_CENTER_EMPIRICAL) */
 
 /* ---- status codes ------------------------------------------------------ */
@@ -94,6 +94,36 @@ extern "C" {
                          FP64 path to ~1e-6 (bound tested: 1e-5, BASELINE north_star "optional FP32
                          path").  Applies where the tensor-core harmonic kernel does (dense
                          METROLOGY-table entry points, harmonic evaluator); ignored elsewhere. */
+
+#define GPPD_COVARIANCE 0x100u /* (= 256) the statistical uncertainty of every fit: after the
+                               fit, one extra streaming pass (csrc/cov_kernels.cu, FP64 whatever
+                               GPPD_FP32 says) forms the Gauss-Newton covariance of the REPORTED
+                               parameters at the reported values; gppd_covariances returns it.
+                               Nothing else a call returns changes.  Definition, per fit:
+                                 model  m_n = c + a p_n exp(j b s_n),  p_n = power_state FCphasor_n,
+                                        s_n = sin(fl(fl(omega t_n) + phi)), cs_n = cos of the same
+                                        rounded argument, weight w_n (1 in bright mode); n runs over
+                                        the job's valid rows (onlyhigh, TRANSIENT), N_valid of them
+                                 theta  = (c.re, c.im, a.re, a.im, b, phi) in params order; without
+                                        GPPD_FITOFFSETS the model has no c: k = 4 and rows / columns
+                                        0-1 of the result are 0 (k = 6 otherwise)
+                                 J_n    = dm/dtheta = (1, j, g, j g, j a s g, j a b cs g),
+                                        g = p e^{j b s}
+                                 H      = Re sum w conj(J_n) J_n^T  (k x k)
+                                 s^2    = sum w |m_n - d_n|^2 / (2 N_valid - k)
+                                 cov    = s^2 H^-1
+                               evaluated at the exported (b, phi) (after the sign normalisation
+                               b < 0 -> -b, phi +- pi), so that entries pairing b with another
+                               parameter have the sign of the reported parametrisation.  All 36
+                               entries of a fit are NaN when 2 N_valid <= k, when the Cholesky
+                               factorisation of the diagonally scaled H meets a pivot <= 1e-12,
+                               when the fit's group is outside group_mask, or when the fit itself
+                               has a NaN.  In ellipse mode it is the covariance of the fit to the
+                               corrected channels (the maps are treated as exact).  With this flag
+                               a batch of the table entry points runs as one launch sequence
+                               (gppd_set_split_chains has no effect), so that every fit's result
+                               is on the slot gppd_covariances reads. */
+#define GPPD_COV_STRIDE 36    /* doubles per fit: a 6 x 6 matrix, row-major */
 
 /* which evaluator computes chi2(b, phi) inside the fit */
 #define GPPD_METHOD_AUTO 0     /* harmonic when its validity conditions hold, else direct */
@@ -360,6 +390,14 @@ int gppd_centres(gppd_handle h, int slot, int64_t ntables, double *centres);
  */
 #define GPPD_ELLIPSE_STRIDE 6
 int gppd_ellipses(gppd_handle h, int slot, int64_t ntables, double *ell, int32_t *status);
+
+/*
+ * The parameter covariances (GPPD_COVARIANCE) of the last call on pipeline slot `slot`:
+ * cov [nfits][6][6] in params order (table, then window, then diode).  GPPD_ERR_ARG when
+ * that call ran without the flag or had fewer than nfits fits.  Waits like gppd_centres;
+ * after gppd_file_submit, call it once gppd_file_wait has returned.
+ */
+int gppd_covariances(gppd_handle h, int slot, int64_t nfits, double *cov);
 
 /*
  * Test hook: the harmonic-sum table of the last batch of pipeline slot `slot`

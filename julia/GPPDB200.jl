@@ -37,6 +37,8 @@ const GPPD_CENTER_EMPIRICAL = UInt32(32)
 const GPPD_FP32        = UInt32(64)   # optional reduced-precision harmonic sums (off by default)
 const GPPD_CENTER_ELLIPSE = UInt32(128)   # `--center ellipse`: offset + ellipse correction per channel
 const GPPD_ELLIPSE_STRIDE = 6
+const GPPD_COVARIANCE  = UInt32(0x100)   # parameter covariances of every fit (gppd_covariances)
+const GPPD_COV_STRIDE  = 36
 
 # struct gppd_options (include/gppd.h)
 struct Options
@@ -306,6 +308,21 @@ function ellipses(slot::Integer = 0)
     gppd_assert_ok(ccall((:gppd_ellipses, libgppd), Cint, (Ptr{Cvoid}, Cint, Int64, Ptr{Float64}, Ptr{Int32}),
                          gethandle(), slot, 1, ell, status))
     return ell, status
+end
+
+"""
+    gppd_covariances(nfits, slot = 0) -> Array{Float64,3}
+
+The parameter covariances of the last call on `slot` made with `GPPD_COVARIANCE` in its
+flags: a 6 x 6 x nfits array, `cov[:, :, f]` the covariance of fit f (params order: table,
+window, diode) over (c.re, c.im, a.re, a.im, b, phi).  Symmetric, so Julia's column-major
+view of the C row-major matrices is the same matrix.
+"""
+function gppd_covariances(nfits::Integer, slot::Integer = 0)
+    cov = Array{Float64,3}(undef, 6, 6, nfits)
+    gppd_assert_ok(ccall((:gppd_covariances, libgppd), Cint, (Ptr{Cvoid}, Cint, Int64, Ptr{Float64}),
+                         gethandle(), slot, nfits, cov))
+    return cov
 end
 
 end # module
